@@ -14,7 +14,10 @@ every rank renders its block with no further communication, and ONE NCCL gather 
 mask to rank 0.  `--scaling weak` renders a whole frame on every rank (N frames per step) instead; at
 N > 1 the strong line carries the weak measurement as `weak_scaling`.  At N = 1 both are the same job.
 
-Prints ONE JSON line on rank 0.
+The headline, end-to-end and extra lines each time --steps steps (the per-kernel profiling pass at most 2).
+Prints ONE JSON line on rank 0.  `--dump-outputs DIR` also writes the frame the last headline step rendered
+(rgb / depth / mask, float32 .npy): the inputs are seeded, so two builds run with the same arguments can be
+compared output for output.
 """
 
 import argparse
@@ -59,7 +62,30 @@ def parse():
                        "of memory', config.py:168; results do not depend on it)")
   ap.add_argument("--view-kernel", default="default", choices=["default", "twin", "quad", "pipe"],
                   help="per-view stage kernel: library default, twin-warp, quad schedule, or sub-round pipelined twin")
-  return ap.parse_args()
+  ap.add_argument("--dump-outputs", metavar="DIR",
+                  help="after the timed steps, write the frame the last headline step rendered as DIR/{rgb,depth,mask}.npy")
+  a = ap.parse_args()
+  if a.steps < 1:
+    ap.error("--steps must be at least 1")
+  return a
+
+
+DUMP_CAP_BYTES = 64 << 20
+
+
+def dump_outputs(path, px, cap_bytes=DUMP_CAP_BYTES):
+  """Writes one rendered frame, [rays, 5] = the rgb / depth / mask of render_rays_mv's outputs_fine_ref, as float32
+  DIR/rgb.npy [N, 3], depth.npy [N], mask.npy [N].  A frame above `cap_bytes` is cut to a fixed seeded sample of
+  rays (in ray order), so that two builds run with the same arguments write the same rays."""
+  import numpy as np
+  px = px.detach().float().cpu()
+  keep = cap_bytes // (px.shape[1] * 4)
+  if px.shape[0] > keep:
+    idx = torch.randperm(px.shape[0], generator=torch.Generator().manual_seed(0))[:keep].sort().values
+    px = px[idx]
+  os.makedirs(path, exist_ok=True)
+  for name, v in (("rgb", px[:, 0:3]), ("depth", px[:, 3]), ("mask", px[:, 4])):
+    np.save(os.path.join(path, name + ".npy"), np.ascontiguousarray(v.numpy(), dtype=np.float32))
 
 
 def peaks():
@@ -357,20 +383,21 @@ def main():
       return n
 
   def timed(fn, steps):
+    """(ms of `steps` calls of fn, what the last call returned)"""
     if world > 1:
       dist.barrier()
     torch.cuda.synchronize()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(steps):
-      fn()
+      out = fn()
     e1.record()
     torch.cuda.synchronize()
     ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
     if world > 1:
       dist.barrier()
       dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-    return ms.item()
+    return ms.item(), out
 
   flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)
   fr = Frame(a.scaling)
@@ -382,12 +409,12 @@ def main():
   sampler = ClockSampler(local)
   sampler.start()
   _lib.lib.dyn_launch_count(1)
-  ms = timed(fr.step_resident, a.steps)
+  ms, px_last = timed(fr.step_resident, a.steps)
   launches = int(_lib.lib.dyn_launch_count(0))
   clocks = sampler.finish()
   # ---- end to end: pinned host buffers in, pinned host pixels out, every step ----
   fr.step_e2e()
-  ms_e2e = timed(fr.step_e2e, a.steps)
+  ms_e2e, _ = timed(fr.step_e2e, a.steps)
   h2d = torch.tensor([float(fr.h2d_bytes())], device=dev)
   d2h = torch.tensor([float(fr.out_host.numel() * fr.out_host.element_size())], device=dev)
   if world > 1:
@@ -399,7 +426,7 @@ def main():
   if not a.no_extras:
     prof_steps = min(a.steps, 2)
     _lib.lib.dyn_profile_enable(1)
-    ms_prof = timed(fr.step_resident, prof_steps)
+    ms_prof, _ = timed(fr.step_resident, prof_steps)
     for cls, name in enumerate(KERNEL_CLASSES):
       tot, n = ctypes.c_float(), ctypes.c_int()
       _lib.check(_lib.lib.dyn_profile_read(cls, ctypes.byref(tot), ctypes.byref(n)))
@@ -412,7 +439,7 @@ def main():
     fw = Frame("weak")
     for _ in range(2):
       fw.step_resident()
-    ms_w = timed(fw.step_resident, a.steps)
+    ms_w, _ = timed(fw.step_resident, a.steps)
     extras["weak_scaling"] = {"value": a.rays * world * a.steps / (ms_w / 1e3), "unit": "rays/s",
                               "ms_per_step": ms_w / a.steps, "note": "every rank renders a whole frame"}
     del fw
@@ -422,15 +449,21 @@ def main():
     fe = Frame(a.scaling, 7, 11)
     for _ in range(2):
       fe.step_resident()
-    ms_e = timed(fe.step_resident, 2)
+    ms_e, _ = timed(fe.step_resident, a.steps)
     fpr_e = flops.flop_per_ray(w["N_samples"], w["N_samples"] + w["N_importance"], 7, 11)
-    extras["eval_shape"] = {"views": "7 dynamic + 11 static", "value": a.rays * 2 / (ms_e / 1e3), "unit": "rays/s",
-                            "ms_per_step": ms_e / 2, "flop_per_ray": fpr_e,
-                            "tflops": a.rays * 2 / (ms_e / 1e3) * fpr_e / 1e12}
+    extras["eval_shape"] = {"views": "7 dynamic + 11 static", "value": a.rays * a.steps / (ms_e / 1e3),
+                            "unit": "rays/s", "ms_per_step": ms_e / a.steps, "flop_per_ray": fpr_e,
+                            "tflops": a.rays * a.steps / (ms_e / 1e3) * fpr_e / 1e12}
     del fe
 
   if not a.no_extras and world == 1:
-    extras["train_step"] = train_step_line(dev, a.precision)
+    extras["train_step"] = train_step_line(dev, a.precision, steps=a.steps)
+
+  if a.dump_outputs:
+    if world > 1 and a.scaling == "strong":  # rank 0's block -> the whole frame on rank 0
+      px_last = dd.gather_pixels(px_last, fr.n_total)
+    if rank == 0:
+      dump_outputs(a.dump_outputs, px_last)
 
   total_rays = fr.n_total * a.steps
   value = total_rays / (ms / 1e3)

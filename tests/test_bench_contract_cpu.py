@@ -7,6 +7,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -54,6 +55,30 @@ def test_oracle_ref_is_the_unmodified_reference_when_built():
   ref = build_ref.load()
   assert ref.rr.__file__.endswith(os.path.join("oracle", "_ref", "ibrnet", "render_ray.pyc"))
   assert callable(ref.rr.render_rays_mv) and callable(ref.ri.render_single_image_nvi)
+
+
+def test_dump_outputs_writes_the_frame_as_float32_arrays(tmp_path):
+  sys.path.insert(0, ROOT)
+  import bench
+  px = torch.randn(40, 5, generator=torch.Generator().manual_seed(0))
+  bench.dump_outputs(str(tmp_path / "full"), px)
+  got = {n: np.load(tmp_path / "full" / (n + ".npy")) for n in ("rgb", "depth", "mask")}
+  assert all(v.dtype == np.float32 for v in got.values())
+  np.testing.assert_array_equal(got["rgb"], px[:, 0:3].numpy())
+  np.testing.assert_array_equal(got["depth"], px[:, 3].numpy())
+  np.testing.assert_array_equal(got["mask"], px[:, 4].numpy())
+  # above the size cap: the same seeded sample of rays, kept in ray order, on every call
+  for d in ("a", "b"):
+    bench.dump_outputs(str(tmp_path / d), px, cap_bytes=10 * 5 * 4)
+  a, b = (np.load(tmp_path / d / "rgb.npy") for d in ("a", "b"))
+  np.testing.assert_array_equal(a, b)
+  rows = [int(np.flatnonzero((px[:, 0:3].numpy() == r).all(1))[0]) for r in a]
+  assert a.shape == (10, 3) and rows == sorted(rows)
+
+
+def test_steps_must_be_positive():
+  p = _run("--steps", "0")
+  assert p.returncode != 0 and "--steps" in p.stderr
 
 
 def test_product_arm_fails_loudly_without_cuda():

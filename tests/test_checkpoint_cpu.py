@@ -1,6 +1,6 @@
 """Checkpoint ingest (row f4): dicts / files in the reference's save layout (ibrnet/model.py:177-232,
 :424-468) load strictly into the parameter containers, reproduce the flat parameter blob the CUDA library
-packs, and -- in the build container -- checkpoints written from the REFERENCE's own nn.Modules load too."""
+packs, and checkpoints laid out as the REFERENCE's own nn.Modules write them load too."""
 
 import os
 from types import SimpleNamespace
@@ -62,18 +62,20 @@ def test_strict_loading_rejects_a_wrong_layout():
     dmodel.model_from_checkpoints(args, coarse=coarse)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/ibrnet"),
-                    reason="live reference only exists in the build container")
 def test_checkpoint_written_by_the_reference_modules_loads():
-  from oracle import build_ref
-  if not build_ref.available():
-    build_ref.build()
-  ref = build_ref.load()
+  """State dicts laid out exactly as the reference's own modules write them: names, order, shapes and dtypes
+  (tests/golden/checkpoint_layout.pt from make_golden_checks.py), filled with seeded values."""
+  layout = torch.load(os.path.join(os.path.dirname(__file__), "golden", "checkpoint_layout.pt"), weights_only=False)
+  g = torch.Generator().manual_seed(3)
+
+  def state_dict(entries):
+    return {name: torch.randn(shape, generator=g).to(getattr(torch, dtype.split(".")[1]))
+            for name, shape, dtype in entries}
+
   args = _args()
-  torch.manual_seed(3)
-  fine = {"net_fine_st": ref.mlp.DynibarStatic(args, 32, 32).state_dict(),
-          "net_fine_dy": ref.mlp.DynibarDynamic(args, 32, 32).state_dict(),
-          "motion_mlp_fine": ref.mlp.MotionMLP(num_basis=6).state_dict(),
+  fine = {"net_fine_st": state_dict(layout["net_fine_st"]),
+          "net_fine_dy": state_dict(layout["net_fine_dy"]),
+          "motion_mlp_fine": state_dict(layout["motion_mlp_fine"]),
           "traj_basis_fine": dmodel.init_dct_basis(6, 24), "global_step": 7}
   got, info = dmodel.model_from_checkpoints(args, fine=fine)
   for key, name in (("net_fine_st", "net_fine_st"), ("net_fine_dy", "net_fine_dy"), ("motion_mlp_fine", "motion_mlp_fine")):

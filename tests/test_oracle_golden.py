@@ -1,11 +1,8 @@
 """Pin the CPU oracle (oracle/dynibar_oracle.py) against the reference.
 
-1. against the committed golden fixtures (outputs of the unmodified reference,
-   tests/golden/make_golden.py) -- runs anywhere;
-2. against the live reference when /root/reference is present (build container).
+Against committed golden fixtures: outputs of the unmodified reference
+(tests/golden/make_golden.py, make_golden_checks.py).
 """
-
-import os
 
 import pytest
 import torch
@@ -127,25 +124,22 @@ def test_sample_pdf_edge_cases():
   torch.testing.assert_close(s[0], torch.linspace(0, 1, 16), atol=1e-5, rtol=0)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/ibrnet"),
-                    reason="live reference only exists in the build container")
-def test_oracle_matches_live_reference():
-  from golden import make_golden as mg
-  ref = mg.import_reference()
-  cfg = dict(scenes.GOLDEN_CONFIGS["mv_small"], seed=77, rays=16, V_dy=7, V_st=4)
+def test_oracle_matches_live_reference(golden):
+  """A scene none of the other fixtures uses (seed 77, 7 + 4 views), against the reference's render_rays_mv
+  (tests/golden/mv_seed77.pt from make_golden_checks.py)."""
+  fx = golden("mv_seed77")
+  cfg = fx["cfg"]
+  assert cfg == dict(scenes.GOLDEN_CONFIGS["mv_small"], seed=77, rays=16, V_dy=7, V_st=4)
   batch, feat_c, feat_f, frame, t, offs, model, args = scenes.build(cfg)
-  mref = mg.reference_model(ref, model, args, False)
+  assert abs(_checksum(batch, [feat_c, feat_f]) - fx["checksum"]) < 1e-6 * fx["checksum"]
   with torch.no_grad():
-    want = ref.rr.render_rays_mv(frame, t, offs, batch, mref, ref.proj.Projector("cpu"),
-                                 feat_c, feat_f, cfg["N_samples"], args,
-                                 inv_uniform=True, N_importance=cfg["N_importance"],
-                                 det=True, is_train=False)
     got = orc.render_rays_mv(frame, t, offs, batch, model, None, feat_c, feat_f,
                              cfg["N_samples"], args, inv_uniform=True,
                              N_importance=cfg["N_importance"], det=True, is_train=False)
   for k in ("outputs_coarse_ref", "outputs_fine_ref", "outputs_fine_ref_dy"):
-    for kk in want[k]:
-      _cmp("%s/%s" % (k, kk), got[k][kk], want[k][kk])
+    assert list(got[k].keys()) == list(fx[k].keys()), k
+    for kk in fx[k]:
+      _cmp("%s/%s" % (k, kk), got[k][kk], fx[k][kk])
 
 
 def test_oracle_encoder_matches_reference_fixture(golden):

@@ -1,6 +1,6 @@
 """RaySamplerSingleImage (row a1) against outputs of the unmodified reference class
-(ibrnet/sample_ray.py:19-331; fixture tests/golden/sampler.pt from make_golden_frame.py) and,
-in the build container, against the live reference."""
+(ibrnet/sample_ray.py:19-331; fixtures tests/golden/sampler.pt from make_golden_frame.py and
+sampler_17x23.pt from make_golden_checks.py)."""
 
 import os
 
@@ -54,17 +54,16 @@ def test_random_sample_matches_reference_fixture():
     s.sample_random_pixel(4, "nope")
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/ibrnet"),
-                    reason="live reference only exists in the build container")
 def test_sampler_matches_live_reference():
-  from golden import make_golden as mg
-  ref = mg.import_reference()
-  cfg = dict(scenes.GOLDEN_CONFIGS["mv_small"], H=17, W=23, rays=None, seed=91)
+  """A 17x23 frame at render_stride 1 and 3 (tests/golden/sampler_17x23.pt from make_golden_checks.py)."""
+  fx = torch.load(os.path.join(os.path.dirname(__file__), "golden", "sampler_17x23.pt"), weights_only=False)
+  cfg = fx["cfg"]
+  assert cfg == dict(scenes.GOLDEN_CONFIGS["mv_small"], H=17, W=23, rays=None, seed=91)
   batch = scenes.build(cfg)[0]
   data = scenes.sampler_data(batch, cfg["H"], cfg["W"], cfg["seed"])
   for stride in (1, 3):
     a = sr.RaySamplerSingleImage(data, "cpu", render_stride=stride).get_all()
-    b = ref.sr.RaySamplerSingleImage(data, "cpu", render_stride=stride).get_all()
+    b = fx[stride]
     for k, w in b.items():
       if torch.is_tensor(w):
         torch.testing.assert_close(a[k], w, rtol=1e-6, atol=1e-6)
