@@ -106,8 +106,8 @@ size_t dyn_net_param_count(int kind) {
 
 size_t dyn_net_packed_bytes(int kind) {
   switch (kind) {
-    case DYN_NET_DYNAMIC: return (size_t)dynamic_layout().all.packed_bytes + view_twin_bytes(kind) + view_quad_bytes(kind) + view_twin3_bytes(kind) + fused_chain_bytes(kind) + twin_chain_bytes(kind);
-    case DYN_NET_STATIC: return (size_t)static_layout(true).all.packed_bytes + view_twin_bytes(kind) + view_quad_bytes(kind) + view_twin3_bytes(kind) + fused_chain_bytes(kind) + twin_chain_bytes(kind);
+    case DYN_NET_DYNAMIC: return (size_t)dynamic_layout().all.packed_bytes + view_twin3_bytes(kind) + twin_chain_bytes(kind);
+    case DYN_NET_STATIC: return (size_t)static_layout(true).all.packed_bytes + view_twin3_bytes(kind) + twin_chain_bytes(kind);
     case DYN_NET_MOTION: return (size_t)motion_layout(8).all.packed_bytes + fused_chain_bytes(kind);
     default: return 0;
   }
@@ -187,17 +187,13 @@ int dyn_net_create_ex(int kind, const float* params, size_t n_params, void* pack
       if (e == cudaSuccess) e = cudaStreamSynchronize((cudaStream_t)stream);
       int rc = e == cudaSuccess ? DYN_OK : fail(DYN_E_CUDA, "reading parameters back: %s", cudaGetErrorString(e));
       char* cur = reinterpret_cast<char*>(packed) + ll.packed_bytes;
-      if (!rc && kind != DYN_NET_MOTION) {
-        rc = view_twin_build(n, hp, cur, view_twin_bytes(kind), (cudaStream_t)stream);
-        cur += view_twin_bytes(kind);
-        if (!rc) rc = view_quad_build(n, hp, cur, view_quad_bytes(kind), (cudaStream_t)stream);
-        cur += view_quad_bytes(kind);
-        if (!rc) rc = view_twin3_build(n, hp, cur, view_twin3_bytes(kind), (cudaStream_t)stream);
+      if (!rc && kind == DYN_NET_MOTION) {
+        rc = fused_chain_build(n, hp, cur, fused_chain_bytes(kind), (cudaStream_t)stream);
+      } else if (!rc) {
+        rc = view_twin3_build(n, hp, cur, view_twin3_bytes(kind), (cudaStream_t)stream);
         cur += view_twin3_bytes(kind);
+        if (!rc) rc = twin_chain_build(n, hp, cur, twin_chain_bytes(kind), (cudaStream_t)stream);
       }
-      if (!rc) rc = fused_chain_build(n, hp, cur, fused_chain_bytes(kind), (cudaStream_t)stream);
-      cur += fused_chain_bytes(kind);
-      if (!rc) rc = twin_chain_build(n, hp, cur, twin_chain_bytes(kind), (cudaStream_t)stream);
       free(hp);
       if (rc) { free(n); return rc; }
     }

@@ -1,7 +1,7 @@
 // Ray-transformer attention on tcgen05 (a11: ibrnet/mlp_network.py:13-31, :84-98).
 //
 // One CTA = one 128-row tile = 128/S whole rays (S | 128).  Q, K, V arrive as bf16 tile
-// images (fused_engine.cuh; written by point1_fused_kernel) and are landed in shared memory
+// images (fused_engine.cuh; written by point1_twin_kernel) and are landed in shared memory
 // by bulk copies (K, V: 32 KB each per tile; Q: one 8 KB head slice at a time);
 // per head h:  logits = Q_h K_h^T  (UMMA 128x128x32, fp32 in TMEM columns [0,128))
 //              softmax over the keys of the row's own ray, in registers

@@ -1,17 +1,12 @@
-// Fused tcgen05 MLP chains that are row-local (no cross-row reduction inside the
-// chain), built on fused_engine.cuh:
+// The MotionMLP as one fused tcgen05 chain (row-local: no cross-row reduction inside it), built on
+// fused_engine.cuh:
 //
-//   motion_fused_kernel : MotionMLP, PE(xyzt) -> 8 x (256, ReLU) with skip -> 18 coeffs
+//   motion_fused_kernel : PE(xyzt) -> 8 x (256, ReLU) with skip -> 18 coeffs
 //                         (mlp_network.py:605-618 + render_ray.py:459-472)
-//   point1_fused_kernel : geometry_fc -> (+ sinusoid) -> Q | K | V projections
-//                         (mlp_network.py:283-286 / :496, :84-86)
-//   point2_fused_kernel : attention fc + residual + LayerNorm -> heads
-//                         (mlp_network.py:99-102, :291-315 / :503-506, first rgb_fc layer)
-//   rgbhead_fused_kernel: static per-view colour-blending head + masked softmax over views
-//                         (mlp_network.py:508-526)
 //
-// All use 256 rows per iteration (two M=128 UMMA tiles), one row per thread in
-// warps 0-7, the MMA issuer in warp 8 and the weight producer in warp 9.
+// 256 rows per iteration (two M=128 UMMA tiles), one row per thread in warps 0-7, the MMA issuer in
+// warp 8 and the weight producer in warp 9.  The aggregation nets' row-local chains are in chains_twin.cu.
+// Also here: the host-only unit-test hooks behind dyn_debug_pack_layer / dyn_debug_tile_image_off.
 #include "fused_engine.cuh"
 #include "nets.cuh"
 
@@ -52,20 +47,15 @@ __device__ __forceinline__ void wait_acc(uint32_t bar0, int bt, uint32_t& acc_cn
   tc_fence_after_sync();
 }
 
-template <int ACT>  // 0 none, 1 ELU, 2 ReLU
-__device__ __forceinline__ void epi_cols_to_A(uint8_t* arow, uint32_t tacc, int ncols, const float* bias) {
+// ReLU(acc + bias) of `ncols` accumulator columns -> bf16 operand columns [0, ncols)
+__device__ __forceinline__ void relu_cols_to_A(uint8_t* arow, uint32_t tacc, int ncols, const float* bias) {
 #pragma unroll 1
   for (int cb = 0; cb < ncols; cb += 32) {
     float acc[32];
     tmem_ld32(tacc + cb, acc);
     tmem_wait_ld();
 #pragma unroll
-    for (int i = 0; i < 32; ++i) {
-      float v = acc[i] + bias[cb + i];
-      if (ACT == 1) v = elu_fast(v);
-      if (ACT == 2) v = fmaxf(v, 0.f);
-      acc[i] = v;
-    }
+    for (int i = 0; i < 32; ++i) acc[i] = fmaxf(acc[i] + bias[cb + i], 0.f);
 #pragma unroll
     for (int g = 0; g < 4; ++g) store8(arow, cb + 8 * g, acc + 8 * g);
   }
@@ -143,7 +133,7 @@ __global__ void __launch_bounds__(320, 1) motion_fused_kernel(const __grid_const
       operand_ready(bar0, bt);
       for (int l = 0; l < 5; ++l) {  // pts_linears.0 .. 4
         wait_acc(bar0, bt, acc_cnt);
-        epi_cols_to_A<2>(arow, tacc, 256, cst + 256 * l);
+        relu_cols_to_A(arow, tacc, 256, cst + 256 * l);
         operand_ready(bar0, bt);
       }
       // pts_linears.5 on cat([input_pts, h]): h part consumed first, then the
@@ -153,7 +143,7 @@ __global__ void __launch_bounds__(320, 1) motion_fused_kernel(const __grid_const
       operand_ready(bar0, bt);
       for (int l = 5; l < 8; ++l) {  // epilogues of pts_linears.5 .. 7
         wait_acc(bar0, bt, acc_cnt);
-        epi_cols_to_A<2>(arow, tacc, 256, cst + 256 * l);
+        relu_cols_to_A(arow, tacc, 256, cst + 256 * l);
         operand_ready(bar0, bt);
       }
       // coeff_linear (18 of 32 columns), zero the last samples of each ray
@@ -168,431 +158,6 @@ __global__ void __launch_bounds__(320, 1) motion_fused_kernel(const __grid_const
         for (int i = 0; i < 32; ++i)
           if (i < a.ncoef) dst[i] = zero ? 0.f : (acc[i] + cst[2048 + i]);
       }
-      tc_fence_before_sync();
-    }
-  }
-  fused_teardown(tmem_base);
-}
-
-// ---------------------------------------------------------------------------
-// per-point stage 1: G -> geometry_fc -> (+ posenc) -> g2, Q, K, V
-// ---------------------------------------------------------------------------
-__global__ void __launch_bounds__(320, 1) point1_fused_kernel(const __grid_constant__ Point1Args a) {
-  constexpr bool kPP = true;
-  extern __shared__ __align__(1024) uint8_t smem[];
-  uint8_t* ring = smem + 2 * kATileBytes;
-  float* cst = reinterpret_cast<float*>(ring + kRing * kStageBytes);  // b_geo0[256] b_geo2[128]
-  uint64_t* bars = reinterpret_cast<uint64_t*>(cst + 2304);
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 14);
-  const int tid = threadIdx.x, warp = tid >> 5;
-  const uint32_t bar0 = smem_u32(bars);
-  __shared__ __align__(16) FusedChunk s_tab[kMaxChunks];
-  stage_chunks(s_tab, a.chunks, a.nchunks);
-  for (int i = tid; i < 256; i += blockDim.x) cst[i] = a.params[a.o_bgeo0 + i];
-  for (int i = tid; i < 128; i += blockDim.x) cst[256 + i] = a.params[a.o_bgeo2 + i];
-  if (tid == 0) { mbar_init(bar0 + 8u * 12, 1); mbar_init(bar0 + 8u * 13, 1); }
-  const uint32_t tmem_base = fused_prologue(bars, tmem_slot, kPP);
-  const int n_iter = (int)((a.P + 255) / 256);
-
-  if (warp == 9) {
-    if ((tid & 31) < a.producers) producer_loop<kPP>(s_tab, a.nchunks, a.wimg, n_iter, ring, bar0, tid & 31, a.producers);
-  } else if (warp == 8) {
-    issuer_loop<kPP>(s_tab, a.nchunks, n_iter, smem, ring, bar0, tmem_base);
-  } else {
-    const int tile = tid >> 7, r = tid & 127;
-    const int bt = kPP ? tile : 0;
-    uint8_t* arow = smem + tile * kATileBytes + (r >> 3) * 128 + (r & 7) * 16;
-    const uint32_t tacc = tmem_addr(tmem_base, (uint32_t)((warp & 3) * 32), (uint32_t)(tile * 256));
-    uint32_t acc_cnt = 0, g_cnt = 0;
-    const uint32_t gbar = bar0 + 8u * (12 + tile);  // this tile's G block has landed
-    const uint8_t* gimg = reinterpret_cast<const uint8_t*>(a.G);
-    const uint32_t atile = smem_u32(smem + tile * kATileBytes);
-    auto issue_g = [&](int it2) {
-      mbar_arrive_expect_tx(gbar, (uint32_t)kATileBytes);
-      bulk_g2s(atile, gimg + ((size_t)it2 * 2 + tile) * (size_t)kATileBytes, (uint32_t)kATileBytes, gbar);
-    };
-    if (r == 0 && (int)blockIdx.x < n_iter) issue_g((int)blockIdx.x);
-    for (int it = blockIdx.x; it < n_iter; it += gridDim.x) {
-      const long long row = (long long)it * 256 + tid;
-      const bool valid = row < a.P;
-      // operand: the pooled statistics G arrive as a ready-made tile image (written by the
-      // per-view kernel): one 68 KB bulk copy per 128 points, issued one iteration ahead
-      mbar_wait(gbar, g_cnt & 1); ++g_cnt;
-      operand_ready(bar0, bt);
-      wait_acc(bar0, bt, acc_cnt);  // geometry_fc.0
-      epi_cols_to_A<1>(arow, tacc, 256, cst);
-      operand_ready(bar0, bt);
-      wait_acc(bar0, bt, acc_cnt);  // geometry_fc.2 (+ sinusoid for the dynamic net) -> g2
-      {
-        const int s_idx = valid ? (int)(row % a.S) : 0;
-#pragma unroll 1
-        for (int cb = 0; cb < 128; cb += 32) {
-          float acc[32];
-          tmem_ld32(tacc + cb, acc);
-          tmem_wait_ld();
-#pragma unroll
-          for (int i = 0; i < 32; ++i) {
-            float v = elu_fast(acc[i] + cst[256 + cb + i]);
-            if (a.posenc) v += __ldg(a.posenc + s_idx * 128 + cb + i);
-            acc[i] = v;
-          }
-          if (valid) {  // residual stream, fp32 tile layout (fused_engine.cuh: tile_f32_off)
-            uint8_t* o = reinterpret_cast<uint8_t*>(a.g2) + tile_f32_off(row, cb >> 2);
-#pragma unroll
-            for (int i = 0; i < 8; ++i)
-              *reinterpret_cast<float4*>(o + i * 2048) = make_float4(acc[4 * i], acc[4 * i + 1], acc[4 * i + 2], acc[4 * i + 3]);
-          }
-#pragma unroll
-          for (int g = 0; g < 4; ++g) store8(arow, cb + 8 * g, acc + 8 * g);
-        }
-      }
-      operand_ready(bar0, bt);
-      wait_acc(bar0, bt, acc_cnt);  // [Wq ; Wk] (N = 256, no bias) -> bf16 rows (operands of the attention)
-#pragma unroll 1
-      for (int cb = 0; cb < 256; cb += 32) {
-        float acc[32];
-        tmem_ld32(tacc + cb, acc);
-        tmem_wait_ld();
-        {  // Q / K as bf16 tile images (16 k-groups), the attention kernel's operands; rows past
-           // the last point are written as zeros (the attention reads whole 128-row tiles)
-          if (!valid) {
-#pragma unroll
-            for (int i = 0; i < 32; ++i) acc[i] = 0.f;
-          }
-          uint8_t* o = reinterpret_cast<uint8_t*>(cb < 128 ? a.Q : a.K) + tile_image_off(row, (cb & 127) >> 3, 16);
-#pragma unroll
-          for (int i = 0; i < 4; ++i)
-            *reinterpret_cast<uint4*>(o + i * 2048) = make_uint4(pack_bf16x2(acc[8 * i], acc[8 * i + 1]), pack_bf16x2(acc[8 * i + 2], acc[8 * i + 3]),
-                              pack_bf16x2(acc[8 * i + 4], acc[8 * i + 5]), pack_bf16x2(acc[8 * i + 6], acc[8 * i + 7]));
-        }
-      }
-      tc_fence_before_sync();
-      mbar_arrive(bar_aready(bar0, bt));  // operand unchanged; accumulators are free again
-      wait_acc(bar0, bt, acc_cnt);     // Wv
-      if (r == 0 && it + (int)gridDim.x < n_iter) issue_g(it + (int)gridDim.x);  // operand tile is free
-#pragma unroll 1
-      for (int cb = 0; cb < 128; cb += 32) {
-        float acc[32];
-        tmem_ld32(tacc + cb, acc);
-        tmem_wait_ld();
-        {
-          if (!valid) {
-#pragma unroll
-            for (int i = 0; i < 32; ++i) acc[i] = 0.f;
-          }
-          uint8_t* o = reinterpret_cast<uint8_t*>(a.V) + tile_image_off(row, cb >> 3, 16);
-#pragma unroll
-          for (int i = 0; i < 4; ++i)
-            *reinterpret_cast<uint4*>(o + i * 2048) = make_uint4(pack_bf16x2(acc[8 * i], acc[8 * i + 1]), pack_bf16x2(acc[8 * i + 2], acc[8 * i + 3]),
-                              pack_bf16x2(acc[8 * i + 4], acc[8 * i + 5]), pack_bf16x2(acc[8 * i + 6], acc[8 * i + 7]));
-        }
-      }
-      tc_fence_before_sync();
-    }
-  }
-  fused_teardown(tmem_base);
-}
-
-// ---------------------------------------------------------------------------
-// per-point stage 2: fc(O) + g2 -> LayerNorm -> heads
-// constants: [0,128) ln_w  [128,256) ln_b  [256,512) b_refpts0  [512,640) b_refpts2
-//            [640,768) b_outgeo0  [768,896) w_outgeo2  [896,1024) b_rgb0 (dyn) / b_rgb0 (static GW)
-//            [1024,1088) b_rgb2  [1088,1280) w_rgb4 (3 x 64)  [1280..] misc: b_outgeo2, b_rgb4[3]
-// ---------------------------------------------------------------------------
-template <bool DYNAMIC>
-__global__ void __launch_bounds__(320, 1) point2_fused_kernel(const __grid_constant__ Point2Args a) {
-  constexpr bool kPP = true;
-  extern __shared__ __align__(1024) uint8_t smem[];
-  uint8_t* ring = smem + 2 * kATileBytes;
-  float* cst = reinterpret_cast<float*>(ring + kRing * kStageBytes);
-  uint64_t* bars = reinterpret_cast<uint64_t*>(cst + 2304);
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 14);
-  const int tid = threadIdx.x, warp = tid >> 5;
-  const uint32_t bar0 = smem_u32(bars);
-  __shared__ __align__(16) FusedChunk s_tab[kMaxChunks];
-  stage_chunks(s_tab, a.chunks, a.nchunks);
-  {
-    const float* p = a.params;
-    for (int i = tid; i < 128; i += blockDim.x) {
-      cst[i] = p[a.o_lnw + i]; cst[128 + i] = p[a.o_lnb + i];
-      cst[640 + i] = p[a.o_boutgeo0 + i]; cst[768 + i] = p[a.o_woutgeo2 + i];
-      cst[896 + i] = p[a.o_brgb0 + i];
-      if (DYNAMIC) cst[512 + i] = p[a.o_brefpts2 + i];
-    }
-    if (DYNAMIC) {
-      for (int i = tid; i < 256; i += blockDim.x) cst[256 + i] = p[a.o_brefpts0 + i];
-      for (int i = tid; i < 64; i += blockDim.x) cst[1024 + i] = p[a.o_brgb2 + i];
-      for (int i = tid; i < 192; i += blockDim.x) cst[1088 + i] = p[a.o_wrgb4 + i];
-      if (tid < 3) cst[1281 + tid] = p[a.o_brgb4 + tid];
-    }
-    if (tid == 0) {
-      cst[1280] = p[a.o_boutgeo2];
-      mbar_init(bar0 + 8u * 12, 1);
-      mbar_init(bar0 + 8u * 13, 1);
-    }
-  }
-  const uint32_t tmem_base = fused_prologue(bars, tmem_slot, kPP);
-  const int n_iter = (int)((a.P + 255) / 256);
-
-  if (warp == 9) {
-    if ((tid & 31) < a.producers) producer_loop<kPP>(s_tab, a.nchunks, a.wimg, n_iter, ring, bar0, tid & 31, a.producers);
-  } else if (warp == 8) {
-    issuer_loop<kPP>(s_tab, a.nchunks, n_iter, smem, ring, bar0, tmem_base);
-  } else {
-    const int tile = tid >> 7, r = tid & 127;
-    const int bt = kPP ? tile : 0;
-    uint8_t* arow = smem + tile * kATileBytes + (r >> 3) * 128 + (r & 7) * 16;
-    const uint32_t tacc = tmem_addr(tmem_base, (uint32_t)((warp & 3) * 32), (uint32_t)(tile * 256));
-    uint32_t acc_cnt = 0, o_cnt = 0;
-    const uint32_t obar = bar0 + 8u * (12 + tile);
-    const uint8_t* oimg = reinterpret_cast<const uint8_t*>(a.O);
-    const uint32_t atile = smem_u32(smem + tile * kATileBytes);
-    auto issue_o = [&](int it2) {
-      mbar_arrive_expect_tx(obar, 32768u);
-      bulk_g2s(atile, oimg + ((size_t)it2 * 2 + tile) * 32768u, 32768u, obar);
-    };
-    if (r == 0 && (int)blockIdx.x < n_iter) issue_o((int)blockIdx.x);
-    for (int it = blockIdx.x; it < n_iter; it += gridDim.x) {
-      const long long row = (long long)it * 256 + tid;
-      const bool valid = row < a.P;
-      // operand: attention output O, a bf16 tile image: one 32 KB bulk copy per 128 points
-      mbar_wait(obar, o_cnt & 1); ++o_cnt;
-      operand_ready(bar0, bt);
-      wait_acc(bar0, bt, acc_cnt);  // fc (no bias) + residual, LayerNorm (eps 1e-6) via TMEM scratch
-      {
-        float sum = 0.f, sq = 0.f;
-#pragma unroll 1
-        for (int cb = 0; cb < 128; cb += 32) {
-          float acc[32];
-          tmem_ld32(tacc + cb, acc);
-          tmem_wait_ld();
-          const uint8_t* res = reinterpret_cast<const uint8_t*>(a.g2) + tile_f32_off(row, cb >> 2);
-#pragma unroll
-          for (int i = 0; i < 8; ++i) {
-            float4 q = valid ? __ldg(reinterpret_cast<const float4*>(res + i * 2048)) : make_float4(0.f, 0.f, 0.f, 0.f);
-            acc[4 * i] += q.x; acc[4 * i + 1] += q.y; acc[4 * i + 2] += q.z; acc[4 * i + 3] += q.w;
-          }
-#pragma unroll
-          for (int i = 0; i < 32; ++i) { sum += acc[i]; sq = fmaf(acc[i], acc[i], sq); }
-          tmem_st32(tacc + 128 + cb, acc);
-        }
-        tmem_wait_st();
-        const float mean = sum * (1.f / 128.f);
-        const float var = fmaxf(sq * (1.f / 128.f) - mean * mean, 0.f);
-        const float rstd = rsqrtf(var + 1e-6f);
-#pragma unroll 1
-        for (int cb = 0; cb < 128; cb += 32) {
-          float y[32];
-          tmem_ld32(tacc + 128 + cb, y);
-          tmem_wait_ld();
-#pragma unroll
-          for (int i = 0; i < 32; ++i) y[i] = (y[i] - mean) * rstd * cst[cb + i] + cst[128 + cb + i];
-#pragma unroll
-          for (int g = 0; g < 4; ++g) store8(arow, cb + 8 * g, y + 8 * g);
-        }
-      }
-      if (DYNAMIC) {
-        // append PE(pts) (33) at columns 128..160, zero to 176 (ref_pts_fc input)
-        float p3[3] = {0.f, 0.f, 0.f};
-        if (valid) { p3[0] = a.pts[row * 3]; p3[1] = a.pts[row * 3 + 1]; p3[2] = a.pts[row * 3 + 2]; }
-        float pe[48];
-        pe_pow2<3, 5>(p3, pe);
-#pragma unroll
-        for (int i = 33; i < 48; ++i) pe[i] = 0.f;
-#pragma unroll
-        for (int g = 0; g < 6; ++g) store8(arow, 128 + 8 * g, pe + 8 * g);
-        operand_ready(bar0, bt);
-        wait_acc(bar0, bt, acc_cnt);  // ref_pts_fc.0
-        epi_cols_to_A<1>(arow, tacc, 256, cst + 256);
-        operand_ready(bar0, bt);
-        wait_acc(bar0, bt, acc_cnt);  // ref_pts_fc.2 -> g4; append PE(dir) (27) at 128..154
-        epi_cols_to_A<1>(arow, tacc, 128, cst + 512);
-        {
-          const long long ray = valid ? row / a.S : 0;
-          float d3[3] = {a.ray_dir[ray * 3], a.ray_dir[ray * 3 + 1], a.ray_dir[ray * 3 + 2]};
-          float pe2[32];
-          pe_pow2<3, 4>(d3, pe2);
-#pragma unroll
-          for (int i = 27; i < 32; ++i) pe2[i] = 0.f;
-#pragma unroll
-          for (int g = 0; g < 4; ++g) store8(arow, 128 + 8 * g, pe2 + 8 * g);
-        }
-      }
-      operand_ready(bar0, bt);
-      // round: out_geometry_fc.0 -> cols [0,128), rgb_fc.0 (dyn) / rgb_fc.0[:, :128] (static) -> [128,256)
-      wait_acc(bar0, bt, acc_cnt);
-      float sigma = cst[1280];
-#pragma unroll 1
-      for (int cb = 0; cb < 128; cb += 32) {
-        float acc[32];
-        tmem_ld32(tacc + cb, acc);
-        tmem_wait_ld();
-#pragma unroll
-        for (int i = 0; i < 32; ++i)
-          sigma = fmaf(elu_fast(acc[i] + cst[640 + cb + i]), cst[768 + cb + i], sigma);
-      }
-      const float nv = valid ? a.nvalid[row] : 0.f;
-      if (!DYNAMIC && r == 0 && it + (int)gridDim.x < n_iter) issue_o(it + (int)gridDim.x);  // last MMA round is done
-      if (DYNAMIC) {
-        epi_cols_to_A<1>(arow, tacc + 128, 128, cst + 896);  // ELU(rgb_fc.0) -> operand
-        operand_ready(bar0, bt);
-        wait_acc(bar0, bt, acc_cnt);  // rgb_fc.2 (64) -> rgb_fc.4 (3) as dot products
-        if (r == 0 && it + (int)gridDim.x < n_iter) issue_o(it + (int)gridDim.x);
-        float c3[3] = {cst[1281], cst[1282], cst[1283]};
-#pragma unroll 1
-        for (int cb = 0; cb < 64; cb += 32) {
-          float acc[32];
-          tmem_ld32(tacc + cb, acc);
-          tmem_wait_ld();
-#pragma unroll
-          for (int i = 0; i < 32; ++i) {
-            const float h = elu_fast(acc[i] + cst[1024 + cb + i]);
-            c3[0] = fmaf(h, cst[1088 + cb + i], c3[0]);
-            c3[1] = fmaf(h, cst[1088 + 64 + cb + i], c3[1]);
-            c3[2] = fmaf(h, cst[1088 + 128 + cb + i], c3[2]);
-          }
-        }
-        if (valid) {
-          const bool none = nv < 1.f;  // mlp_network.py:297-299, :314
-          reinterpret_cast<float4*>(a.raw)[row] =
-              make_float4(none ? 0.f : sigmoid_fast(c3[0]), none ? 0.f : sigmoid_fast(c3[1]),
-                          none ? 0.f : sigmoid_fast(c3[2]), none ? -1e9f : sigma - a.shift);
-        }
-      } else {
-        // static: per-point part of the blending head, GW = rgb_fc.0[:, :128] g + b, and sigma
-#pragma unroll 1
-        for (int cb = 0; cb < 128; cb += 32) {
-          float acc[32];
-          tmem_ld32(tacc + 128 + cb, acc);
-          tmem_wait_ld();
-          if (valid) {  // fp32 tile layout, read per (point, view) row by the blending head
-            uint8_t* o = reinterpret_cast<uint8_t*>(a.GW) + tile_f32_off(row, cb >> 2);
-#pragma unroll
-            for (int i = 0; i < 8; ++i)
-              *reinterpret_cast<float4*>(o + i * 2048) = make_float4(acc[4 * i] + cst[896 + cb + 4 * i], acc[4 * i + 1] + cst[896 + cb + 4 * i + 1],
-                                 acc[4 * i + 2] + cst[896 + cb + 4 * i + 2], acc[4 * i + 3] + cst[896 + cb + 4 * i + 3]);
-          }
-        }
-        if (valid) a.sigma[row] = nv < 1.f ? -1e9f : sigma;
-      }
-      tc_fence_before_sync();
-    }
-  }
-  fused_teardown(tmem_base);
-}
-
-// ---------------------------------------------------------------------------
-// static colour-blending head (per (point, view) rows, VP view slots per point)
-// constants: [0,128) unused  [128,192) b_rgb2  [192,256) w_rgb4  [256] b_rgb4
-// ---------------------------------------------------------------------------
-template <int VP>
-__global__ void __launch_bounds__(320, 1) rgbhead_fused_kernel(const __grid_constant__ RgbHeadArgs a) {
-  constexpr bool kPP = true;
-  extern __shared__ __align__(1024) uint8_t smem[];
-  uint8_t* ring = smem + 2 * kATileBytes;
-  float* cst = reinterpret_cast<float*>(ring + kRing * kStageBytes);
-  uint64_t* bars = reinterpret_cast<uint64_t*>(cst + 2304);
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 14);
-  const int tid = threadIdx.x, warp = tid >> 5;
-  const uint32_t bar0 = smem_u32(bars);
-  __shared__ __align__(16) FusedChunk s_tab[kMaxChunks];
-  stage_chunks(s_tab, a.chunks, a.nchunks);
-  for (int i = tid; i < 64; i += blockDim.x) {
-    cst[128 + i] = a.params[a.o_brgb2 + i];
-    cst[192 + i] = a.params[a.o_wrgb4 + i];
-  }
-  if (tid == 0) {
-    cst[256] = a.params[a.o_brgb4];
-    mbar_init(bar0 + 8u * 12, 1);
-    mbar_init(bar0 + 8u * 13, 1);
-  }
-  const uint32_t tmem_base = fused_prologue(bars, tmem_slot, kPP);
-  const int n_iter = (int)((a.P * VP + 255) / 256);
-
-  if (warp == 9) {
-    if ((tid & 31) < a.producers) producer_loop<kPP>(s_tab, a.nchunks, a.wimg, n_iter, ring, bar0, tid & 31, a.producers);
-  } else if (warp == 8) {
-    issuer_loop<kPP>(s_tab, a.nchunks, n_iter, smem, ring, bar0, tmem_base);
-  } else {
-    const int tile = tid >> 7, r = tid & 127;
-    const int bt = kPP ? tile : 0;
-    uint8_t* arow = smem + tile * kATileBytes + (r >> 3) * 128 + (r & 7) * 16;
-    const uint32_t tacc = tmem_addr(tmem_base, (uint32_t)((warp & 3) * 32), (uint32_t)(tile * 256));
-    const int v = tid % VP;
-    uint32_t acc_cnt = 0, x_cnt = 0;
-    const uint32_t xbar = bar0 + 8u * (12 + tile);  // x block of this tile has landed
-    const uint8_t* ximg = reinterpret_cast<const uint8_t*>(a.X);
-    const uint32_t atile = smem_u32(smem + tile * kATileBytes);
-    auto issue_x = [&](int it2) {
-      mbar_arrive_expect_tx(xbar, 32768u);
-      bulk_g2s(atile, ximg + ((size_t)it2 * 2 + tile) * 32768u, 32768u, xbar);
-    };
-    if (r == 0 && (int)blockIdx.x < n_iter) issue_x((int)blockIdx.x);
-    for (int it = blockIdx.x; it < n_iter; it += gridDim.x) {
-      const long long pl = ((long long)it * 256 + tid) / VP;
-      const bool pt_ok = pl < a.P;
-      const bool valid = pt_ok && v < a.V;
-      const long long m = pl * a.V + v;
-      // operand: [x (128) | vis2, ray_diff (4) | 0 ...] = 144 columns; the x block is the tile image
-      // spilled by the per-view kernel and arrives by bulk copy (issued one iteration ahead)
-      {
-        float t[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-        if (valid) {
-          const float4 rd = __ldg(reinterpret_cast<const float4*>(a.ray_diff) + m);
-          t[0] = a.vis2[m]; t[1] = rd.x; t[2] = rd.y; t[3] = rd.z; t[4] = rd.w;
-        }
-        store8(arow, 128, t);
-        float z[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-        store8(arow, 136, z);
-      }
-      mbar_wait(xbar, x_cnt & 1); ++x_cnt;
-      operand_ready(bar0, bt);
-      wait_acc(bar0, bt, acc_cnt);  // rgb_fc.0: per-view part + per-point part GW (bias folded into GW)
-      // the MMA has consumed columns [0,144): prefetch the next iteration's x block behind it
-      // (the hidden layer below goes to columns [144,272) of the same tile)
-      if (r == 0 && it + (int)gridDim.x < n_iter) issue_x(it + (int)gridDim.x);
-#pragma unroll 1
-      for (int cb = 0; cb < 128; cb += 32) {
-        float acc[32];
-        tmem_ld32(tacc + cb, acc);
-        tmem_wait_ld();
-        const uint8_t* gw = reinterpret_cast<const uint8_t*>(a.GW) + tile_f32_off(pt_ok ? pl : 0, cb >> 2);
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-          const float4 q = __ldg(reinterpret_cast<const float4*>(gw + i * 2048));
-          acc[4 * i] = elu_fast(acc[4 * i] + q.x); acc[4 * i + 1] = elu_fast(acc[4 * i + 1] + q.y);
-          acc[4 * i + 2] = elu_fast(acc[4 * i + 2] + q.z); acc[4 * i + 3] = elu_fast(acc[4 * i + 3] + q.w);
-        }
-#pragma unroll
-        for (int g = 0; g < 4; ++g) store8(arow, 144 + cb + 8 * g, acc + 8 * g);
-      }
-      operand_ready(bar0, bt);
-      wait_acc(bar0, bt, acc_cnt);  // rgb_fc.2 (64, ELU) -> rgb_fc.4 logit
-      float logit = cst[256];
-#pragma unroll 1
-      for (int cb = 0; cb < 64; cb += 32) {
-        float acc[32];
-        tmem_ld32(tacc + cb, acc);
-        tmem_wait_ld();
-#pragma unroll
-        for (int i = 0; i < 32; ++i)
-          logit = fmaf(elu_fast(acc[i] + cst[128 + cb + i]), cst[192 + cb + i], logit);
-      }
-      // masked softmax over the views of the point, blend source colours (mlp_network.py:523-525)
-      const float mk = valid ? a.mask_eff[m] : 0.f;
-      float l = valid ? (mk == 0.f ? -1e9f : logit) : -INFINITY;
-      float mx = l;
-      mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, 1));
-      mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, 2));
-      mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, 4));
-      if (VP == 16) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, 8));
-      const float e = valid ? __expf(l - mx) : 0.f;
-      const float den = group_sum<VP>(e);
-      const float w = e / den;
-      float c0 = 0.f, c1 = 0.f, c2 = 0.f;
-      if (valid) { c0 = a.rgb_in[m * 3] * w; c1 = a.rgb_in[m * 3 + 1] * w; c2 = a.rgb_in[m * 3 + 2] * w; }
-      c0 = group_sum<VP>(c0); c1 = group_sum<VP>(c1); c2 = group_sum<VP>(c2);
-      if (pt_ok && v == 0) reinterpret_cast<float4*>(a.raw)[pl] = make_float4(c0, c1, c2, a.sigma[pl]);
       tc_fence_before_sync();
     }
   }
@@ -663,145 +228,52 @@ int debug_pack_layer(const float* W, const float* bias, int N, int Kw, int Npad,
 }
 size_t debug_tile_image_off(long long row, int kgroup, int kgroups) { return tile_image_off(row, kgroup, kgroups); }
 
-size_t fused_chain_bytes(int kind) {
-  return kind == DYN_NET_MOTION ? (size_t)(1280 * 1024) : (size_t)(768 * 1024);
-}
+size_t fused_chain_bytes(int kind) { return kind == DYN_NET_MOTION ? (size_t)(1280 * 1024) : 0; }
 
 int fused_chain_build(dyn_net* n, const float* P, void* dst_dev, size_t dst_bytes, cudaStream_t st) {
+  if (n->kind != DYN_NET_MOTION) return DYN_OK;
   std::vector<uint8_t> img;
   std::vector<FusedChunk> tab;
   char* cur = reinterpret_cast<char*>(dst_dev);
   size_t left = dst_bytes;
   int rc = DYN_OK;
-  auto add = [&](const LinearP& l, int row0, int N, int Npad, int Kpad, std::vector<int> map, int d_col = 0,
-                 int a_kg0 = 0, int first_flags = 9, bool last = true) {
+  auto add = [&](const LinearP& l, int N, int Npad, int Kpad, std::vector<int> map, int first_flags = 9) {
     HostLayer L;
-    L.W = P + l.w + (size_t)row0 * l.in; L.N = N; L.Kw = l.in; L.Npad = Npad; L.Kpad = Kpad;
+    L.W = P + l.w; L.N = N; L.Kw = l.in; L.Npad = Npad; L.Kpad = Kpad;
     L.colmap = std::move(map);
-    append_layer(L, img, tab, d_col, a_kg0, first_flags, last);
+    append_layer(L, img, tab, 0, 0, first_flags, true);
   };
-  if (n->kind == DYN_NET_MOTION) {
-    const MotionLayout& L = n->ml;
-    // operand order: k-major [cos f_k (4) | sin f_k (4)] x 16, then x(4): weight column of each
-    std::vector<int> pe(144, -1);
-    for (int k = 0; k < 16; ++k)
-      for (int d = 0; d < 4; ++d) { pe[8 * k + d] = 4 + 4 * k + d; pe[8 * k + 4 + d] = 68 + 4 * k + d; }
-    for (int d = 0; d < 4; ++d) pe[128 + d] = d;
-    add(L.pts[0], 0, 256, 256, 144, pe);
-    for (int i = 1; i < 5; ++i) add(L.pts[i], 0, 256, 256, 256, identity_map(256, 256));
-    {  // pts_linears.5: input cat([pe(132), h(256)]) -> h part first, then the pe part accumulates
-      std::vector<int> hmap(256);
-      for (int i = 0; i < 256; ++i) hmap[i] = 132 + i;
-      add(L.pts[5], 0, 256, 256, 256, hmap, 0, 0, 9, true);
-      add(L.pts[5], 0, 256, 256, 144, pe, 0, 0, 1, true);  // wait for the re-filled operand, accumulate
-    }
-    add(L.pts[6], 0, 256, 256, 256, identity_map(256, 256));
-    add(L.pts[7], 0, 256, 256, 256, identity_map(256, 256));
-    add(L.coeff, 0, 3 * n->nb, 32, 256, identity_map(256, 256));
-    upload(img, tab, cur, left, &n->chain[0], st, &rc);
-    return rc;
+  const MotionLayout& L = n->ml;
+  // operand order: k-major [cos f_k (4) | sin f_k (4)] x 16, then x(4): weight column of each
+  std::vector<int> pe(144, -1);
+  for (int k = 0; k < 16; ++k)
+    for (int d = 0; d < 4; ++d) { pe[8 * k + d] = 4 + 4 * k + d; pe[8 * k + 4 + d] = 68 + 4 * k + d; }
+  for (int d = 0; d < 4; ++d) pe[128 + d] = d;
+  add(L.pts[0], 256, 256, 144, pe);
+  for (int i = 1; i < 5; ++i) add(L.pts[i], 256, 256, 256, identity_map(256, 256));
+  {  // pts_linears.5: input cat([pe(132), h(256)]) -> h part first, then the pe part accumulates
+    std::vector<int> hmap(256);
+    for (int i = 0; i < 256; ++i) hmap[i] = 132 + i;
+    add(L.pts[5], 256, 256, 256, hmap);
+    add(L.pts[5], 256, 256, 144, pe, 1);  // wait for the re-filled operand, accumulate
   }
-  const bool dynamic = n->kind == DYN_NET_DYNAMIC;
-  const LinearP &geo0 = dynamic ? n->dl.geo0 : n->sl.geo0, &geo2 = dynamic ? n->dl.geo2 : n->sl.geo2;
-  const LinearP &wq = dynamic ? n->dl.wq : n->sl.wq, &wk = dynamic ? n->dl.wk : n->sl.wk;
-  const LinearP &wv = dynamic ? n->dl.wv : n->sl.wv, &fc = dynamic ? n->dl.fc : n->sl.fc;
-  const LinearP &og0 = dynamic ? n->dl.outgeo0 : n->sl.outgeo0;
-  const LinearP &rgb0 = dynamic ? n->dl.rgb0 : n->sl.rgb0;
-  // ---- point stage 1: geo0 (K 257 -> 272), geo2, [Wq;Wk] (two 128-row halves of one N=256 layer), Wv
-  add(geo0, 0, 256, 256, 272, identity_map(257, 272));
-  add(geo2, 0, 128, 128, 256, identity_map(256, 256));
-  {
-    // [Wq ; Wk]: build a temporary stacked weight [256,128]
-    std::vector<float> qk(256 * 128);
-    memcpy(qk.data(), P + wq.w, 128 * 128 * sizeof(float));
-    memcpy(qk.data() + 128 * 128, P + wk.w, 128 * 128 * sizeof(float));
-    HostLayer L;
-    L.W = qk.data(); L.N = 256; L.Kw = 128; L.Npad = 256; L.Kpad = 128; L.colmap = identity_map(128, 128);
-    append_layer(L, img, tab);
-  }
-  add(wv, 0, 128, 128, 128, identity_map(128, 128));
-  upload(img, tab, cur, left, &n->chain[0], st, &rc);
-  if (rc) return rc;
-  // ---- point stage 2
-  add(fc, 0, 128, 128, 128, identity_map(128, 128));
-  if (dynamic) {
-    add(n->dl.refpts0, 0, 256, 256, 176, identity_map(161, 176));
-    add(n->dl.refpts2, 0, 128, 128, 256, identity_map(256, 256));
-    add(og0, 0, 128, 128, 128, identity_map(128, 128), 0, 0, 9, false);
-    add(rgb0, 0, 128, 128, 160, identity_map(155, 160), 128, 0, 8, true);  // same operand, cols [128,256)
-    add(n->dl.rgb2, 0, 64, 64, 128, identity_map(128, 128));
-  } else {
-    add(og0, 0, 128, 128, 128, identity_map(128, 128), 0, 0, 9, false);
-    add(rgb0, 0, 128, 128, 128, identity_map(128, 128), 128, 0, 8, true);  // rgb_fc.0[:, :128] (per-point part)
-  }
-  upload(img, tab, cur, left, &n->chain[1], st, &rc);
-  if (rc) return rc;
-  if (!dynamic) {
-    // ---- static blending head: operand [x 128 | vis2, ray_diff 4 | pad] <-> rgb_fc.0 columns 128..260
-    std::vector<int> m(144, -1);
-    for (int i = 0; i < 133; ++i) m[i] = 128 + i;
-    add(rgb0, 0, 128, 128, 144, m);
-    add(n->sl.rgb2, 0, 64, 64, 128, identity_map(128, 128), 0, 18);  // hidden layer at columns [144,272)
-    upload(img, tab, cur, left, &n->chain[2], st, &rc);
-  }
+  add(L.pts[6], 256, 256, 256, identity_map(256, 256));
+  add(L.pts[7], 256, 256, 256, identity_map(256, 256));
+  add(L.coeff, 3 * n->nb, 32, 256, identity_map(256, 256));
+  upload(img, tab, cur, left, &n->motion, st, &rc);
   return rc;
 }
 
 int launch_motion_fused(const dyn_net* n, MotionFusedArgs& a, cudaStream_t st) {
   a.producers = producer_lanes();
-  if (!n->chain[0].img) return fail(DYN_E_INVALID, "motion net has no fused images");
-  a.wimg = n->chain[0].img; a.chunks = n->chain[0].tab; a.nchunks = n->chain[0].nchunks;
+  if (!n->motion.img) return fail(DYN_E_INVALID, "motion net has no fused images");
+  a.wimg = n->motion.img; a.chunks = n->motion.tab; a.nchunks = n->motion.nchunks;
   a.params = n->params;
   for (int i = 0; i < 8; ++i) a.o_bias[i] = n->ml.pts[i].b;
   a.o_bias[8] = n->ml.coeff.b;
   a.ncoef = 3 * n->nb;
   ProfScope prof(PROF_MOTION, st);
   return launch_chain(motion_fused_kernel, a, a.N, st);
-}
-
-int launch_point1_fused(const dyn_net* n, Point1Args& a, cudaStream_t st) {
-  a.producers = producer_lanes();
-  if (!n->chain[0].img) return fail(DYN_E_INVALID, "net has no fused point-stage images");
-  const bool dynamic = n->kind == DYN_NET_DYNAMIC;
-  a.wimg = n->chain[0].img; a.chunks = n->chain[0].tab; a.nchunks = n->chain[0].nchunks;
-  a.params = n->params;
-  a.o_bgeo0 = dynamic ? n->dl.geo0.b : n->sl.geo0.b;
-  a.o_bgeo2 = dynamic ? n->dl.geo2.b : n->sl.geo2.b;
-  ProfScope prof(PROF_POINT1, st);
-  return launch_chain(point1_fused_kernel, a, a.P, st);
-}
-
-int launch_point2_fused(const dyn_net* n, Point2Args& a, cudaStream_t st) {
-  a.producers = producer_lanes();
-  if (!n->chain[1].img) return fail(DYN_E_INVALID, "net has no fused point-stage images");
-  const bool dynamic = n->kind == DYN_NET_DYNAMIC;
-  a.wimg = n->chain[1].img; a.chunks = n->chain[1].tab; a.nchunks = n->chain[1].nchunks;
-  a.params = n->params;
-  a.shift = n->shift;
-  ProfScope prof(PROF_POINT2, st);
-  if (dynamic) {
-    const DynamicLayout& L = n->dl;
-    a.o_lnw = L.ln_w; a.o_lnb = L.ln_b; a.o_brefpts0 = L.refpts0.b; a.o_brefpts2 = L.refpts2.b;
-    a.o_boutgeo0 = L.outgeo0.b; a.o_woutgeo2 = L.outgeo2.w; a.o_boutgeo2 = L.outgeo2.b;
-    a.o_brgb0 = L.rgb0.b; a.o_brgb2 = L.rgb2.b; a.o_wrgb4 = L.rgb4.w; a.o_brgb4 = L.rgb4.b;
-    return launch_chain(point2_fused_kernel<true>, a, a.P, st);
-  }
-  const StaticLayout& L = n->sl;
-  a.o_lnw = L.ln_w; a.o_lnb = L.ln_b; a.o_brefpts0 = 0; a.o_brefpts2 = 0;
-  a.o_boutgeo0 = L.outgeo0.b; a.o_woutgeo2 = L.outgeo2.w; a.o_boutgeo2 = L.outgeo2.b;
-  a.o_brgb0 = L.rgb0.b; a.o_brgb2 = 0; a.o_wrgb4 = 0; a.o_brgb4 = 0;
-  return launch_chain(point2_fused_kernel<false>, a, a.P, st);
-}
-
-int launch_rgbhead_fused(const dyn_net* n, RgbHeadArgs& a, cudaStream_t st) {
-  a.producers = producer_lanes();
-  if (!n->chain[2].img) return fail(DYN_E_INVALID, "static net has no fused blending-head images");
-  a.wimg = n->chain[2].img; a.chunks = n->chain[2].tab; a.nchunks = n->chain[2].nchunks;
-  a.params = n->params;
-  a.o_brgb2 = n->sl.rgb2.b; a.o_wrgb4 = n->sl.rgb4.w; a.o_brgb4 = n->sl.rgb4.b;
-  ProfScope prof(PROF_RGBHEAD, st);
-  if (a.V <= 8) return launch_chain(rgbhead_fused_kernel<8>, a, a.P * 8, st);
-  return launch_chain(rgbhead_fused_kernel<16>, a, a.P * 16, st);
 }
 
 }  // namespace dyn

@@ -1,9 +1,8 @@
-// Row-local fused tcgen05 chains in the twin-warp structure of view_twin.cu: TWO independent CTAs per SM,
-// each with ONE 128-row tile whose rows are served by TWO threads (warps w and w + 4 share the TMEM lane
-// quadrant w & 3 and split every layer's output columns), plus the MMA issuer (warp 8) and the weight
-// producer (warp 9).  The round-1 versions of these kernels (chains_fused.cu: one 320-thread CTA per SM,
-// two tiles, one thread per row) leave only 8 row warps on an SM; here 16 row warps share it and the two
-// CTAs desynchronise, which is what the latency-bound epilogues need (profiles/r02_chain_kernels.md).
+// Row-local fused tcgen05 chains of the aggregation networks in the twin-warp structure of the per-view
+// kernel (view_twin3.cu): TWO independent CTAs per SM, each with ONE 128-row tile whose rows are served by
+// TWO threads (warps w and w + 4 share the TMEM lane quadrant w & 3 and split every layer's output columns),
+// plus the MMA issuer (warp 8) and the weight producer (warp 9).  16 row warps share an SM and the two CTAs
+// desynchronise, which is what the latency-bound epilogues need (profiles/r02_chain_kernels.md).
 //
 //   rgbhead_twin_kernel : static per-view colour-blending head + masked softmax over views
 //                         (mlp_network.py:508-526)
@@ -227,9 +226,6 @@ __device__ __forceinline__ void t_elu_log2_blocks(uint8_t* arow, uint32_t tacc, 
     store8(arow, dst0 + 16 * h, v);
     store8(arow, dst0 + 16 * h + 8, v + 8);
   });
-}
-__device__ __forceinline__ void t_elu_log2_32(uint8_t* arow, uint32_t tacc, int col0, int dst0) {
-  t_elu_log2_blocks<1>(arow, tacc, col0, dst0);
 }
 // NB blocks of 32 accumulator columns -> bf16 tile image rows (16 k-groups: 4 per block starting at kgroup0),
 // zeros for rows past the end

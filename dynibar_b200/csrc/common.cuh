@@ -119,17 +119,12 @@ struct dyn_net {
   dyn::DynamicLayout dl;
   dyn::StaticLayout sl;
   dyn::MotionLayout ml;
-  // row-local fused chains (chains_fused.cu): motion: [0]; aggregation nets:
-  // [0] point stage 1, [1] point stage 2, [2] static blending head
-  dyn::ChainImage chain[3];
-  // the same chains in the twin-warp structure (chains_twin.cu): [0] point stage 1, [1] point stage 2,
+  // motion net: the whole MotionMLP as one fused chain (chains_fused.cu)
+  dyn::ChainImage motion;
+  // aggregation nets, twin-warp row-local chains (chains_twin.cu): [0] point stage 1, [1] point stage 2,
   // [2] static blending head
   dyn::ChainImage chain_tw[3];
-  // twin-warp per-view stage (view_twin.cu): weight images in its column layout
-  dyn::ChainImage twin;
-  // quad-schedule per-view stage (view_quad.cu)
-  dyn::ChainImage quad;
-  // sub-round pipelined twin kernel (view_twin3.cu)
+  // aggregation nets, per-view stage (view_twin3.cu): weight images in its column layout
   dyn::ChainImage twin3;
 };
 

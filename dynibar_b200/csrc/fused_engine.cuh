@@ -1,4 +1,4 @@
-// Shared machinery of the fused tcgen05 kernels (nets_fused.cu, chains_fused.cu):
+// Shared machinery of the fused tcgen05 kernels (view_twin3.cu, chains_twin.cu, chains_fused.cu):
 // smem budget constants, fast activations, A-tile stores, view-group shuffles,
 // the table-driven weight producer and MMA issuer, and the host-side packing of
 // weight chunks into UMMA images.
@@ -16,8 +16,6 @@ using namespace tc;
 constexpr int kRing = 4;
 constexpr int kStageBytes = 16384;
 constexpr int kATileBytes = 69632;  // 128 rows x 272 cols bf16 (34 k-groups: geometry_fc.0 has K = 257)
-constexpr int kConstFloats = 2048;
-constexpr int kSmemFused = 2 * kATileBytes + kRing * kStageBytes + kConstFloats * 4 + 256;
 // barrier slots inside the fused kernels: [0..3] w_full, [4..7] w_empty, [8] a_ready, [9] acc_full
 
 __device__ __forceinline__ float ex2f(float x) {
@@ -77,20 +75,6 @@ __device__ __forceinline__ void store8(uint8_t* arow, int c0, const float* v) {
   q.z = pack_bf16x2(v[4], v[5]);
   q.w = pack_bf16x2(v[6], v[7]);
   *reinterpret_cast<uint4*>(arow + (c0 >> 3) * 2048) = q;
-}
-
-// acc[32] (+bias, ELU) -> bf16 columns [c0, c0+32) of the A tile, optional row scale
-template <bool kElu>
-__device__ __forceinline__ void epi32_to_A(uint8_t* arow, int c0, float* acc, const float* bias,
-                                           float scale) {
-#pragma unroll
-  for (int i = 0; i < 32; ++i) {
-    float v = acc[i] + bias[c0 + i];
-    if (kElu) v = elu_fast(v);
-    acc[i] = v * scale;
-  }
-#pragma unroll
-  for (int g = 0; g < 4; ++g) store8(arow, c0 + 8 * g, acc + 8 * g);
 }
 
 // PE with frequencies 2^k via angle doubling: out = [x(D), cos(2^k x)(NF*D), sin(2^k x)(NF*D)]
@@ -430,21 +414,6 @@ inline void append_layer_plan(const HostLayer& L, std::vector<uint8_t>& img, std
 inline std::vector<int> identity_map(int K, int Kpad) {
   std::vector<int> m(Kpad, -1);
   for (int i = 0; i < K; ++i) m[i] = i;
-  return m;
-}
-// [mean8 | var8 | feat8] per channel group; C channels, source columns
-// [0,C) mean, [C,2C) var, [2C,3C) per-view feature
-inline std::vector<int> pooled_map(int C, int groups, int Kpad) {
-  std::vector<int> m(Kpad, -1);
-  for (int g = 0; g < groups; ++g)
-    for (int j = 0; j < 8; ++j) {
-      const int c = 8 * g + j;
-      if (c < C) {
-        m[24 * g + j] = c;
-        m[24 * g + 8 + j] = C + c;
-        m[24 * g + 16 + j] = 2 * C + c;
-      }
-    }
   return m;
 }
 

@@ -763,7 +763,7 @@ size_t motion_f32_workspace(long long N) {
 int motion_f32(const dyn_net* n, const float* x, int ldx, bool time_is_column, float time,
                long long N_all, float* coeff, void* ws, size_t ws_bytes, int prec, cudaStream_t st) {
   const MotionLayout& L = n->ml;
-  if (prec == DYN_PREC_BF16 && n->chain[0].img != nullptr) {
+  if (prec == DYN_PREC_BF16 && n->motion.img != nullptr) {
     // whole MLP in one tcgen05 kernel (chains_fused.cu); no workspace needed
     MotionFusedArgs a;
     memset(&a, 0, sizeof(a));
@@ -867,8 +867,7 @@ static int run_point_fused(const dyn_net* n, const float* G, long long P, int R,
     DYN_LAUNCH_CHECK();
     p1.posenc = posenc_tab;
   }
-  if (use_twin_chains()) RUN(launch_point1_twin(n, p1, st));
-  else RUN(launch_point1_fused(n, p1, st));
+  RUN(launch_point1_twin(n, p1, st));
   if (attention_tc_supported(S)) {
     RUN(launch_attention_tc(Qb, Kb, Vb, t.nvalid, P, S, Ob, st));
   } else {
@@ -883,8 +882,7 @@ static int run_point_fused(const dyn_net* n, const float* G, long long P, int R,
     DYN_LAUNCH_CHECK();
   }
   p2.O = Ob; p2.g2 = t.G2; p2.nvalid = t.nvalid; p2.P = P; p2.S = S;
-  if (use_twin_chains()) return launch_point2_twin(n, p2, st);
-  return launch_point2_fused(n, p2, st);
+  return launch_point2_twin(n, p2, st);
 }
 
 // unit-test hook: the per-point fused stage on caller-provided G / nvalid
@@ -996,8 +994,7 @@ int net_static_fused(const dyn_net* n, const float* pts, const float* ray_o, con
       memset(&rh, 0, sizeof(rh));
       rh.X = d.X; rh.vis2 = d.vis2; rh.ray_diff = d.rd; rh.mask_eff = d.meff; rh.rgb_in = d.rgbin;
       rh.GW = d.ch; rh.sigma = d.sig; rh.P = P; rh.V = V; rh.raw = raw + p0 * 4;
-      if (use_twin_chains()) RUN(launch_rgbhead_twin(n, rh, st));
-      else RUN(launch_rgbhead_fused(n, rh, st));
+      RUN(launch_rgbhead_twin(n, rh, st));
     }
     (void)prec; (void)M;
   }

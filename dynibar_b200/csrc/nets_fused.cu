@@ -1,6 +1,5 @@
-// Host-side dispatch of the fused per-(point, view) stage of the two aggregation networks: argument
-// block + choice between the twin-warp kernel (view_twin.cu, default) and the quad-schedule kernel
-// (view_quad.cu, kept for comparison).
+// Host-side launch of the fused per-(point, view) stage of the two aggregation networks: argument
+// block, then the sub-round pipelined twin-warp kernel (view_twin3.cu).
 //
 // Reference semantics: ibrnet/projection.py:103-176, ibrnet/mlp_network.py:236-284
 // (dynamic) and :423-497 (static).
@@ -12,30 +11,15 @@
 
 namespace dyn {
 
-constexpr int kDefaultViewKernel = 3;  // sub-round pipelined twin kernel + software-pipelined TMEM read-out (profiles/r02_kernels.md)
-
-// Three schedules of the same per-tile work: 0 = the twin-warp kernel (view_twin.cu: two independent CTAs per
-// SM), 1 = the quad kernel (view_quad.cu: one CTA per SM alternating between two tiles), 2 = the twin-warp
-// kernel with sub-round pipelined layers (view_twin3.cu).  DYN_VIEW_KERNEL=twin|quad|pipe or
-// dyn_debug_set_view_kernel(); profiles/r02_view_kernels.md has the comparison.
+// dyn_debug_set_view_kernel: -1 = the library's kernel.  Any other id (those of the removed comparison
+// variants in particular) makes every fused per-view launch fail, so a measurement that asks for a variant
+// cannot silently time the default under its name.
 static int g_view_kernel = -1;
-void set_view_kernel(int which) { g_view_kernel = (which >= 0 && which <= 3) ? which : -1; }
-static int view_kernel() {
-  if (g_view_kernel < 0) {
-    const char* e = getenv("DYN_VIEW_KERNEL");
-    g_view_kernel = e == nullptr ? kDefaultViewKernel : (e[0] == 'q' ? 1 : (e[0] == 'p' ? 2 : (e[0] == 'e' ? 3 : 0)));
-  }
-  return g_view_kernel;
-}
+void set_view_kernel(int which) { g_view_kernel = which; }
 
-bool use_twin_chains() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("DYN_CHAINS");
-    v = (e != nullptr && e[0] == 'f') ? 0 : 1;
-  }
-  return v == 1;
-}
+// dyn_debug_set_view_kernel ids 0..2 (bench.py --view-kernel twin|quad|pipe)
+static const char* const kRemovedViewKernels[3] = {"round-1 twin-warp kernel ('twin')", "quad-schedule kernel ('quad')",
+                                                   "twin3 without elected arrive ('pipe')"};
 
 int producer_lanes() {
   static int v = -1;
@@ -47,6 +31,12 @@ int producer_lanes() {
 }
 
 int launch_view_fused(const dyn_net* n, ViewFusedArgs& a, int V, cudaStream_t st) {
+  if (g_view_kernel >= 0 && g_view_kernel < 3)
+    return fail(DYN_E_INVALID, "per-view kernel variant %d, the %s, was removed; dyn_debug_set_view_kernel(-1) "
+                "selects the library's kernel", g_view_kernel, kRemovedViewKernels[g_view_kernel]);
+  if (g_view_kernel != -1)
+    return fail(DYN_E_INVALID, "no per-view kernel variant %d; dyn_debug_set_view_kernel(-1) selects the library's "
+                "kernel", g_view_kernel);
   if (V > 16) return fail(DYN_E_INVALID, "fused per-view kernel supports V <= 16 (got %d)", V);
   a.params = n->params;
   a.producers = producer_lanes();
@@ -64,12 +54,7 @@ int launch_view_fused(const dyn_net* n, ViewFusedArgs& a, int V, cudaStream_t st
     a.o_w8 = L.vis2_2.w; a.o_b8 = L.vis2_2.b; a.o_s = -1;
     a.anti_alias = 0; a.mask_rgb = 0;
   }
-  switch (view_kernel()) {
-    case 1: return launch_view_quad(n, a, V, st);
-    case 2: return launch_view_twin3(n, a, V, st, false);
-    case 3: return launch_view_twin3(n, a, V, st, true);  // + one barrier arrival per warp ("elected")
-    default: return launch_view_twin(n, a, V, st);
-  }
+  return launch_view_twin3(n, a, V, st);
 }
 
 }  // namespace dyn

@@ -52,7 +52,7 @@ struct ViewFusedArgs {
   long long* dbg;    // optional: clock64() phase timestamps of block 0 (profiling builds/tests only)
 };
 
-// ---- row-local fused chains (chains_fused.cu) ----
+// ---- row-local fused chains: MotionMLP (chains_fused.cu), point stages and blending head (chains_twin.cu) ----
 struct MotionFusedArgs {
   const float* x;  // [N, ldx] xyz (+ time column when time_is_column)
   int ldx, time_is_column;
@@ -126,32 +126,18 @@ size_t fused_chain_bytes(int kind);
 int fused_chain_build(dyn_net* n, const float* host_params, void* dst_dev, size_t dst_bytes,
                       cudaStream_t st);
 int launch_motion_fused(const dyn_net* n, MotionFusedArgs& a, cudaStream_t st);
-int launch_point1_fused(const dyn_net* n, Point1Args& a, cudaStream_t st);
-int launch_point2_fused(const dyn_net* n, Point2Args& a, cudaStream_t st);
-int launch_rgbhead_fused(const dyn_net* n, RgbHeadArgs& a, cudaStream_t st);
 
-// twin-warp versions of the row-local chains (chains_twin.cu); DYN_CHAINS=fused selects the round-1 kernels
+// twin-warp row-local chains (chains_twin.cu)
 size_t twin_chain_bytes(int kind);
 int twin_chain_build(dyn_net* n, const float* host_params, void* dst_dev, size_t dst_bytes, cudaStream_t st);
 int launch_point1_twin(const dyn_net* n, Point1Args& a, cudaStream_t st);
 int launch_point2_twin(const dyn_net* n, Point2Args& a, cudaStream_t st);
 int launch_rgbhead_twin(const dyn_net* n, RgbHeadArgs& a, cudaStream_t st);
-bool use_twin_chains();
-
-// twin-warp per-view stage (view_twin.cu)
-size_t view_twin_bytes(int kind);
-int view_twin_build(dyn_net* n, const float* host_params, void* dst_dev, size_t dst_bytes, cudaStream_t st);
-int launch_view_twin(const dyn_net* n, ViewFusedArgs& a, int V, cudaStream_t st);
 
 // sub-round pipelined twin-warp per-view stage (view_twin3.cu)
 size_t view_twin3_bytes(int kind);
 int view_twin3_build(dyn_net* n, const float* host_params, void* dst_dev, size_t dst_bytes, cudaStream_t st);
-int launch_view_twin3(const dyn_net* n, ViewFusedArgs& a, int V, cudaStream_t st, bool elected_arrive = false);
-
-// quad-schedule per-view stage (view_quad.cu): one CTA per SM, two tiles, four threads per row
-size_t view_quad_bytes(int kind);
-int view_quad_build(dyn_net* n, const float* host_params, void* dst_dev, size_t dst_bytes, cudaStream_t st);
-int launch_view_quad(const dyn_net* n, ViewFusedArgs& a, int V, cudaStream_t st);
+int launch_view_twin3(const dyn_net* n, ViewFusedArgs& a, int V, cudaStream_t st);
 
 void set_view_kernel(int which);
 int producer_lanes();  // DYN_PRODUCERS (default 1)

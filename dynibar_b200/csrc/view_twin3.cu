@@ -1,7 +1,3 @@
-// Sub-round pipelined version of view_twin.cu (same thread mapping, same math up to the bf16 storage of x):
-// every layer from base_fc.0 on is issued in two sub-rounds so that the tensor cores start on the finished
-// operand columns while the row warps are still in the epilogue of the others (details at "From here on").
-//
 // Fused per-(point, view) stage of the two aggregation networks on tcgen05 (reference:
 // ibrnet/projection.py:103-176, ibrnet/mlp_network.py:236-284 (dynamic) / :423-497 (static)).
 // Per 128-row tile, without leaving the SM:
@@ -15,16 +11,20 @@
 //
 // Engine: fused_engine.cuh (operand tile in shared memory written by the epilogues, accumulators
 // in TMEM, weights streamed through a cp.async.bulk ring, table-driven MMA issuer).  Every row is
-// served by TWO threads in twin warps w and w + 4*NT (same TMEM lane quadrant), which is what the
+// served by TWO threads in twin warps w and w + 4 (same TMEM lane quadrant), which is what the
 // latency-bound epilogues need; each twin owns half of every layer's output columns and half of the
 // gathered / pooled channels, and the twins exchange only two scalars per row and iteration (the
 // partial visibility logits).
 //
-// TWO independent CTAs per SM, each with one 128-row tile:
+// TWO independent CTAs per SM, each with one 128-row tile and a 2-slot weight ring, so the tensor pipe
+// is shared by two unsynchronised instruction streams:
 //   warps 0-3 : twin 0 (quadrant = w & 3)      warps 4-7 : twin 1 of the same rows
 //   warp 8    : MMA issuer (one elected lane)  warp 9    : weight producer
-// (the NT = 2 template value -- one 576-thread CTA with two ping-pong tiles -- was measured 5 % slower in
-// round 1 and is no longer instantiated; the alternating two-tile schedule lives in view_quad.cu).
+//
+// Every layer from base_fc.0 on is issued in two sub-rounds, so the tensor cores start on the finished
+// operand columns while the row warps are still in the epilogue of the others (details at "From here on").
+// The operand barriers count WARPS, not threads (warp_arrive).  The accumulator read-outs are
+// software-pipelined in 16-column halves (fused_engine.cuh: tmem_pipe16).
 //
 // Latency hiding inside a CTA (round 2, profiles/r02_view_kernels.md): the source views are read in
 // their packed per-frame layouts (bf16 channels-last features: 2 x 16-byte loads per tap and twin; RGBA
@@ -44,24 +44,28 @@ using namespace fe;
 
 namespace {
 
-constexpr bool kTwinPP = true;  // ping-pong (measured 8% faster than lock-step, profiles/r01_kernels.md)
 constexpr int kTwinATile = 69632;  // K <= 256 (+ one k-step of bias columns): 34 k-groups
 // T_B5 / T_B7 hold log2(e) * bias, T_W6V / T_W8 hold ln(2) * weight (the hidden activations of vis_fc.0 and
 // vis_fc2.0 live on the exp2 scale); the biases of base_fc.2 and vis_fc.2 ride in the MMA
 constexpr int T_B2 = 0, T_B5 = 48, T_W6V = 176, T_B7 = 304, T_W8 = 432, T_MISC = 560, T_DFEAT = 576,
               T_CAMS = 624 /* 16 views x (P 12 + centre 3 + pad) */, T_XCH = T_CAMS + 256;  // + 2 x [2][128] exchange
 constexpr int kTwinConst = T_XCH + 512;
-// NT = 128-row tiles per CTA: 2 -> one 576-thread CTA per SM (ping-pong between its tiles);
-// 1 -> two independent 320-thread CTAs per SM, each with one tile and a 2-slot weight ring, so
-// the tensor pipe is shared by two unsynchronised instruction streams.
 // weight ring: 16 KB stages; 8 KB stages x twice the slots measured 14 % slower (per-chunk barrier and
 // issue overhead outweighs the faster slot turnover, profiles/r01_kernels.md)
 constexpr int kTwinStage = 16384;
-constexpr int twin_ring(int nt) { return nt == 1 ? 2 : 4; }
-constexpr int twin_smem(int nt) { return nt * kTwinATile + twin_ring(nt) * kTwinStage + kTwinConst * 4 + 256; }
+constexpr int kTwinRing = 2;
+constexpr int kTwinSmem = kTwinATile + kTwinRing * kTwinStage + kTwinConst * 4 + 256;
 
 __device__ __forceinline__ void pair_sync(int pair) {
   asm volatile("bar.sync %0, 64;" ::"r"(pair + 1) : "memory");
+}
+
+// One arrival per warp on an operand barrier: every thread has fenced its own writes (fence.proxy.async +
+// tcgen05.fence::before_thread_sync), the warp converges (__syncwarp orders the lanes' memory operations) and
+// lane 0 arrives once -- 32 same-address shared-memory atomics per warp instruction become one
+__device__ __forceinline__ void warp_arrive(uint32_t bar) {
+  __syncwarp();
+  if ((threadIdx.x & 31) == 0) mbar_arrive(bar);
 }
 
 // 11 values of one PE component: [x, cos(2^k x) k=0..4, sin(2^k x) k=0..4]
@@ -78,48 +82,13 @@ __device__ __forceinline__ void pe_comp(float x, float* o) {
   }
 }
 
-// layers whose bias rides in the MMA and whose accumulator is on the exp2 scale (F1, F3)
-template <int N>
-__device__ __forceinline__ void elu_log2_block_to_A(uint8_t* arow, uint32_t tacc, int col0) {
-#pragma unroll 1
-  for (int cb = 0; cb < N; cb += 32) {
-    float acc[32];
-    tmem_ld32(tacc + col0 + cb, acc);
-    tmem_wait_ld();
-#pragma unroll
-    for (int i = 0; i < 32; ++i) acc[i] = elu_log2(acc[i]);
-#pragma unroll
-    for (int g = 0; g < 4; ++g) store8(arow, col0 + cb + 8 * g, acc + 8 * g);
-  }
-}
-
-template <int N>
-__device__ __forceinline__ void elu_block_to_A(uint8_t* arow, uint32_t tacc, int col0, const float* bias) {
-#pragma unroll 1
-  for (int cb = 0; cb < N; cb += 32) {
-    float acc[32];
-    tmem_ld32(tacc + col0 + cb, acc);
-    tmem_wait_ld();
-#pragma unroll
-    for (int i = 0; i < 32; ++i) acc[i] = elu_fast(acc[i] + bias[col0 + cb + i]);
-#pragma unroll
-    for (int g = 0; g < 4; ++g) store8(arow, col0 + cb + 8 * g, acc + 8 * g);
-  }
-}
-
-// EA ("elected arrive"): the operand barriers count WARPS, not threads: every thread fences its own writes
-// (fence.proxy.async + tcgen05.fence::before_thread_sync), the warp converges (__syncwarp orders the lanes' memory
-// operations) and lane 0 arrives once -- 32 same-address shared-memory atomics per warp instruction become one
-template <int VP, bool ST, int NT, bool EA>
-__global__ void __launch_bounds__(NT * 256 + 64, NT == 1 ? 2 : 1)
-    view_twin3_kernel(const __grid_constant__ ViewFusedArgs a) {
-  constexpr int ROWS = 128 * NT;          // rows per iteration
-  constexpr int RING = twin_ring(NT);
-  constexpr bool PP = (NT == 2) && kTwinPP;
-  constexpr int W_ISSUE = 8 * NT, W_PROD = 8 * NT + 1;
+template <int VP, bool ST>
+__global__ void __launch_bounds__(320, 2) view_twin3_kernel(const __grid_constant__ ViewFusedArgs a) {
+  constexpr int ROWS = 128;  // rows per iteration: one tile
+  constexpr int W_ISSUE = 8, W_PROD = 9;
   extern __shared__ __align__(1024) uint8_t smem[];
-  uint8_t* ring = smem + NT * kTwinATile;
-  float* cst = reinterpret_cast<float*>(ring + RING * kTwinStage);
+  uint8_t* ring = smem + kTwinATile;
+  float* cst = reinterpret_cast<float*>(ring + kTwinRing * kTwinStage);
   uint64_t* bars = reinterpret_cast<uint64_t*>(cst + kTwinConst);
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 24);
   const int tid = threadIdx.x, warp = tid >> 5;
@@ -128,12 +97,12 @@ __global__ void __launch_bounds__(NT * 256 + 64, NT == 1 ? 2 : 1)
   stage_chunks(s_tab, a.chunks, a.nchunks);
 
   if (tid == 0) {
-    init_barriers(bar0, PP, /*arrivals=*/NT == 2 ? 256 : 128, RING);
-    if (NT == 1) {  // second operand barrier (sub-round 1 of the pipelined layers): both twins arrive once
-      mbar_init(bar_aready(bar0, 1, RING), EA ? 8 : 256);
-      if (EA) mbar_init(bar_aready(bar0, 0, RING), 8);
-      mbar_fence_init();
-    }
+    init_barriers(bar0, /*pp=*/false, /*arrivals=*/128, kTwinRing);
+    // both operand barriers count one arrival per row warp (warp_arrive); the second one serves sub-round 1
+    // of the pipelined layers
+    mbar_init(bar_aready(bar0, 1, kTwinRing), 8);
+    mbar_init(bar_aready(bar0, 0, kTwinRing), 8);
+    mbar_fence_init();
   }
   {
     const float* prm = a.params;
@@ -155,7 +124,7 @@ __global__ void __launch_bounds__(NT * 256 + 64, NT == 1 ? 2 : 1)
       cst[T_MISC + 2] = (ST && a.o_s >= 0) ? fabsf(prm[a.o_s]) : 0.f;
     }
   }
-  if (warp == W_ISSUE) tmem_alloc(smem_u32(tmem_slot), 256 * NT);
+  if (warp == W_ISSUE) tmem_alloc(smem_u32(tmem_slot), 256);
   tc_fence_before_sync();
   __syncthreads();
   tc_fence_after_sync();
@@ -166,32 +135,21 @@ __global__ void __launch_bounds__(NT * 256 + 64, NT == 1 ? 2 : 1)
 
   if (warp == W_PROD) {
     if ((tid & 31) < a.producers)
-      producer_loop<PP, RING, kTwinStage>(s_tab, a.nchunks, a.wimg, n_iter, ring, bar0, tid & 31, a.producers);
+      producer_loop<false, kTwinRing, kTwinStage>(s_tab, a.nchunks, a.wimg, n_iter, ring, bar0, tid & 31, a.producers);
   } else if (warp == W_ISSUE) {
-    issuer_loop<PP, NT, RING, kTwinStage>(s_tab, a.nchunks, n_iter, smem, ring, bar0, tmem_base, kTwinATile,
-                           a.dbg ? a.dbg + 128 : nullptr);
+    issuer_loop<false, 1, kTwinRing, kTwinStage>(s_tab, a.nchunks, n_iter, smem, ring, bar0, tmem_base, kTwinATile,
+                                                  a.dbg ? a.dbg + 128 : nullptr);
   } else {
-#define ARRIVE(bar)                                   \
-  do {                                                \
-    if (EA) {                                         \
-      __syncwarp();                                   \
-      if ((tid & 31) == 0) mbar_arrive(bar);          \
-    } else {                                          \
-      mbar_arrive(bar);                               \
-    }                                                 \
-  } while (0)
     const int tw = tid / ROWS;         // twin index
-    const int t = tid % ROWS;          // row slot inside the iteration
-    const int tile = t >> 7, r = t & 127;
-    uint8_t* arow = smem + tile * kTwinATile + (r >> 3) * 128 + (r & 7) * 16;
-    const uint32_t tacc = tmem_addr(tmem_base, (uint32_t)((warp & 3) * 32), (uint32_t)(tile * 256));
+    const int t = tid % ROWS;          // row inside the tile
+    uint8_t* arow = smem + (t >> 3) * 128 + (t & 7) * 16;
+    const uint32_t tacc = tmem_addr(tmem_base, (uint32_t)((warp & 3) * 32), 0u);
     const int v = t % VP;
     const int gl = t & (VP - 1);
-    const int pair = warp & (4 * NT - 1);
-    const int bt = PP ? tile : 0;  // barrier tile
+    const int pair = warp & 3;
+    const uint32_t a_ready = bar_aready(bar0, 0, kTwinRing), acc_full = bar_acc(bar0, 0, kTwinRing);
     float* xch5 = cst + T_XCH;        // [2][128] partial visibility logits of vis_fc
     float* xch7 = cst + T_XCH + 256;  // [2][128] partial logits of vis_fc2
-    static_assert(NT == 1, "exchange arrays are sized for one tile per CTA");
     if (tw == 0) {
       // persistent bias columns of base_fc.2 (K = 256 + 16): k-groups 32, 33 = [1, 1, 0 ...] (hi, lo)
       float o[8] = {1.f, 1.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f}, z[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
@@ -206,8 +164,6 @@ __global__ void __launch_bounds__(NT * 256 + 64, NT == 1 ? 2 : 1)
     if (a.dbg != nullptr && blockIdx.x == 0 && t == 0 && dbg_n < 64)                 \
       a.dbg[tw * 64 + dbg_n++] = clock64();                                             \
   } while (0)
-    constexpr int NG = ST ? 5 : (0);  // static: 5 channel groups per twin (set below for dynamic)
-    (void)NG;
 
     // the first point of this thread; later ones are fetched one iteration ahead (before the last MMA wait)
     float np3[3], nq3[3];
@@ -337,7 +293,7 @@ __global__ void __launch_bounds__(NT * 256 + 64, NT == 1 ? 2 : 1)
         }
         fence_proxy_async_smem();
         tc_fence_before_sync();
-        ARRIVE(bar_aready(bar0, bt, RING));
+        warp_arrive(a_ready);
       }
 
       TS();  // 1: after F1 operand + arrive
@@ -347,7 +303,6 @@ __global__ void __launch_bounds__(NT * 256 + 64, NT == 1 ? 2 : 1)
       for (int i = 0; i < 40; ++i) chv[i] = 0.f;
       float rgb[3] = {0.f, 0.f, 0.f};
       {
-        const int fo = tw == 0 ? 3 : 0;  // twin 0 keeps rgb in slots 0..2
 #pragma unroll
         for (int tp = 0; tp < 4; ++tp) {
           const float wgt = tw4[tp];
@@ -366,7 +321,6 @@ __global__ void __launch_bounds__(NT * 256 + 64, NT == 1 ? 2 : 1)
             }
           }
         }
-        (void)fo;
         if (want_rgb) {
 #pragma unroll
           for (int tp = 0; tp < 4; ++tp) {
@@ -391,22 +345,18 @@ __global__ void __launch_bounds__(NT * 256 + 64, NT == 1 ? 2 : 1)
       TS();  // 2: after gather
       if (ST) {
         // ---- F1 epilogue: this twin's 128 of the 256 columns ----
-        mbar_wait(bar_acc(bar0, bt, RING), acc_cnt & 1); ++acc_cnt;
+        mbar_wait(acc_full, acc_cnt & 1); ++acc_cnt;
         TS();  // 3: F1 acc ready
         tc_fence_after_sync();
-        if (EA) {
-          tmem_pipe16<8>(tacc, [&](int h) { return 128 * tw + 16 * h; }, [&](int h, float* v) {
+        tmem_pipe16<8>(tacc, [&](int h) { return 128 * tw + 16 * h; }, [&](int h, float* v) {
 #pragma unroll
-            for (int i = 0; i < 16; ++i) v[i] = elu_log2(v[i]);
-            store8(arow, 128 * tw + 16 * h, v);
-            store8(arow, 128 * tw + 16 * h + 8, v + 8);
-          });
-        } else {
-          elu_log2_block_to_A<128>(arow, tacc, 128 * tw);
-        }
+          for (int i = 0; i < 16; ++i) v[i] = elu_log2(v[i]);
+          store8(arow, 128 * tw + 16 * h, v);
+          store8(arow, 128 * tw + 16 * h + 8, v + 8);
+        });
         fence_proxy_async_smem();
         tc_fence_before_sync();
-        ARRIVE(bar_aready(bar0, bt, RING));
+        warp_arrive(a_ready);
         TS();  // 4: F1 epilogue done
         // ---- F2: src_feat (35 of 48 columns) * ref_feat; twin 0 keeps 0..17, twin 1 keeps 18..34.
         //      The per-ray reference feature is loaded BEFORE the wait (its L2 latency hides behind the MMA) ----
@@ -416,7 +366,7 @@ __global__ void __launch_bounds__(NT * 256 + 64, NT == 1 ? 2 : 1)
 #pragma unroll
           for (int i = 0; i < 18; ++i) rfv[i] = (tw == 0 || i < 17) ? __ldg(rf + i) : 0.f;
         }
-        mbar_wait(bar_acc(bar0, bt, RING), acc_cnt & 1); ++acc_cnt;
+        mbar_wait(acc_full, acc_cnt & 1); ++acc_cnt;
         TS();  // 5: F2 acc ready
         tc_fence_after_sync();
         float s48[48];
@@ -479,7 +429,7 @@ __global__ void __launch_bounds__(NT * 256 + 64, NT == 1 ? 2 : 1)
           if (ST && g == 2) {
             fence_proxy_async_smem();
             tc_fence_before_sync();
-            ARRIVE(bar_aready(bar0, bt, RING));
+            warp_arrive(a_ready);
           }
         }
         {  // zero the K padding (static: 120..127 / 248..255, dynamic: 120..127)
@@ -490,7 +440,7 @@ __global__ void __launch_bounds__(NT * 256 + 64, NT == 1 ? 2 : 1)
       }
       fence_proxy_async_smem();
       tc_fence_before_sync();
-      ARRIVE(bar_aready(bar0, ST ? 1 : 0, RING));  // static: sub-round 1 of base_fc.0 (second operand barrier)
+      warp_arrive(bar_aready(bar0, ST ? 1 : 0, kTwinRing));  // static: sub-round 1 of base_fc.0 (second operand barrier)
 
       TS();  // 6: pool1 done + arrive
       // From here on every layer runs in TWO sub-rounds: the twins own interleaved 32-column blocks, arrive after
@@ -499,10 +449,10 @@ __global__ void __launch_bounds__(NT * 256 + 64, NT == 1 ? 2 : 1)
       // bf16 in operand columns [0,128) (vis_fc.0 reads it there, vis_fc.2 adds to it), h in [128,256).
       // ---- F3: ELU(base_fc.0): this twin's blocks 4+tw, 6+tw (columns 128..255 first: they free the TMEM half
       //      base_fc.2 accumulates into), then 0+tw, 2+tw ----
-      mbar_wait(bar_acc(bar0, bt, RING), acc_cnt & 1); ++acc_cnt;
+      mbar_wait(acc_full, acc_cnt & 1); ++acc_cnt;
       TS();  // 7: F3 acc ready
       tc_fence_after_sync();
-      if (EA) {
+      {
         auto col3 = [&](int h) { const int j = h >> 1; return 32 * ((j < 2 ? 4 : 0) + 2 * (j & 1) + tw) + 16 * (h & 1); };
         tmem_pipe16<8>(tacc, col3, [&](int h, float* v) {
 #pragma unroll
@@ -512,215 +462,112 @@ __global__ void __launch_bounds__(NT * 256 + 64, NT == 1 ? 2 : 1)
           if ((h & 3) == 3) {
             fence_proxy_async_smem();
             tc_fence_before_sync();
-            ARRIVE(bar_aready(bar0, h >> 2, RING));  // first / second operand barrier
+            warp_arrive(bar_aready(bar0, h >> 2, kTwinRing));  // first / second operand barrier
           }
         });
-      } else {
-#pragma unroll 1
-        for (int j = 0; j < 4; ++j) {
-          const int col = 32 * ((j < 2 ? 4 : 0) + 2 * (j & 1) + tw);
-          elu_log2_block_to_A<32>(arow, tacc, col);
-          if (j & 1) {
-            fence_proxy_async_smem();
-            tc_fence_before_sync();
-            ARRIVE(bar_aready(bar0, j >> 1, RING));  // first / second operand barrier
-          }
-        }
       }
 
       TS();  // 8: F3 epilogue done
       // ---- F4: x = ELU(base_fc.2) (accumulator in TMEM [128,256), bias folded, exp2 scale) -> bf16 operand
       //      columns of this twin's blocks tw, 2 + tw (the pooling weight w1 of vis_fc.0's input is applied to
       //      that layer's accumulator: W (w1 x) = w1 (W x)) ----
-      mbar_wait(bar_acc(bar0, bt, RING), acc_cnt & 1); ++acc_cnt;
+      mbar_wait(acc_full, acc_cnt & 1); ++acc_cnt;
       TS();  // 9: F4 acc ready
       tc_fence_after_sync();
       auto colh = [&](int h) { return 32 * (2 * (h >> 1) + tw) + 16 * (h & 1); };  // this twin's blocks tw, 2 + tw
-      if (EA) {
-        tmem_pipe16<4>(tacc + 128, colh, [&](int h, float* v) {
+      tmem_pipe16<4>(tacc + 128, colh, [&](int h, float* v) {
 #pragma unroll
-          for (int i = 0; i < 16; ++i) v[i] = elu_from_log2(v[i]);
-          store8(arow, colh(h), v);
-          store8(arow, colh(h) + 8, v + 8);
-          if (h & 1) {
-            fence_proxy_async_smem();
-            tc_fence_before_sync();
-            ARRIVE(bar_aready(bar0, h >> 1, RING));
-          }
-        });
-      } else {
-#pragma unroll 1
-        for (int j = 0; j < 2; ++j) {
-          const int cb = 32 * (2 * j + tw);
-          float acc[32];
-          tmem_ld32(tacc + 128 + cb, acc);
-          tmem_wait_ld();
-#pragma unroll
-          for (int i = 0; i < 32; ++i) acc[i] = elu_from_log2(acc[i]);
-#pragma unroll
-          for (int g = 0; g < 4; ++g) store8(arow, cb + 8 * g, acc + 8 * g);
+        for (int i = 0; i < 16; ++i) v[i] = elu_from_log2(v[i]);
+        store8(arow, colh(h), v);
+        store8(arow, colh(h) + 8, v + 8);
+        if (h & 1) {
           fence_proxy_async_smem();
           tc_fence_before_sync();
-          ARRIVE(bar_aready(bar0, j, RING));
+          warp_arrive(bar_aready(bar0, h >> 1, kTwinRing));
         }
-      }
+      });
 
       TS();  // 10: F4 epilogue done
       // ---- F5: h = ELU(w1 (vis_fc.0 x) + b) -> operand columns [128,256); partial visibility logit ----
-      mbar_wait(bar_acc(bar0, bt, RING), acc_cnt & 1); ++acc_cnt;
+      mbar_wait(acc_full, acc_cnt & 1); ++acc_cnt;
       TS();  // 11: F5 acc ready
       tc_fence_after_sync();
       {
         float part = 0.f;
-        if (EA) {
-          tmem_pipe16<4>(tacc, colh, [&](int h, float* v) {
-            const int c0 = colh(h);
+        tmem_pipe16<4>(tacc, colh, [&](int h, float* v) {
+          const int c0 = colh(h);
 #pragma unroll
-            for (int i = 0; i < 16; ++i) {
-              v[i] = elu_log2(fmaf(v[i], w1, cst[T_B5 + c0 + i]));  // log2(e) * ELU(w1 (W x) + b)
-              part = fmaf(v[i], cst[T_W6V + c0 + i], part);
-            }
-            store8(arow, 128 + c0, v);
-            store8(arow, 128 + c0 + 8, v + 8);
-            if (h & 1) {
-              if (h == 3) xch5[tw * 128 + t] = part;
-              fence_proxy_async_smem();
-              tc_fence_before_sync();
-              ARRIVE(bar_aready(bar0, h >> 1, RING));
-            }
-          });
-        } else {
-#pragma unroll 1
-          for (int j = 0; j < 2; ++j) {
-            const int cb = 32 * (2 * j + tw);
-            float acc[32];
-            tmem_ld32(tacc + cb, acc);
-            tmem_wait_ld();
-#pragma unroll
-            for (int i = 0; i < 32; ++i) {
-              acc[i] = elu_log2(fmaf(acc[i], w1, cst[T_B5 + cb + i]));  // log2(e) * ELU(w1 (W x) + b)
-              part = fmaf(acc[i], cst[T_W6V + cb + i], part);
-            }
-#pragma unroll
-            for (int g = 0; g < 4; ++g) store8(arow, 128 + cb + 8 * g, acc + 8 * g);
-            if (j == 1) xch5[tw * 128 + t] = part;
+          for (int i = 0; i < 16; ++i) {
+            v[i] = elu_log2(fmaf(v[i], w1, cst[T_B5 + c0 + i]));  // log2(e) * ELU(w1 (W x) + b)
+            part = fmaf(v[i], cst[T_W6V + c0 + i], part);
+          }
+          store8(arow, 128 + c0, v);
+          store8(arow, 128 + c0 + 8, v + 8);
+          if (h & 1) {
+            if (h == 3) xch5[tw * 128 + t] = part;
             fence_proxy_async_smem();
             tc_fence_before_sync();
-            ARRIVE(bar_aready(bar0, j, RING));
+            warp_arrive(bar_aready(bar0, h >> 1, kTwinRing));
           }
-        }
+        });
       }
 
       TS();  // 12: F5 epilogue done
       // ---- F6: x += ELU(vis_fc.2[:128] h) (accumulator in TMEM [128,256), bias folded); bf16(x) is vis_fc2.0's
       //      operand (vis1 is applied to its accumulator) and, for the static net, the blending head's input ----
-      mbar_wait(bar_acc(bar0, bt, RING), acc_cnt & 1); ++acc_cnt;
+      mbar_wait(acc_full, acc_cnt & 1); ++acc_cnt;
       TS();  // 13: F6 acc ready
       tc_fence_after_sync();
       // both twins arrived on a_ready before this MMA ran: the partial logits are visible
       const float vlogit = cst[T_MISC + 0] + xch5[t] + xch5[128 + t];
       const float vis1 = sigmoid_fast(elu_fast(vlogit)) * mask;
-      if (EA) {
-        tmem_pipe16<4>(tacc + 128, colh, [&](int h, float* v) {
-          const int c0 = colh(h);
-          uint4 pk[2];
+      tmem_pipe16<4>(tacc + 128, colh, [&](int h, float* v) {
+        const int c0 = colh(h);
+        uint4 pk[2];
 #pragma unroll
-          for (int i = 0; i < 2; ++i) {
-            const uint4 q = *reinterpret_cast<const uint4*>(arow + ((c0 >> 3) + i) * 2048);
-            const uint32_t u[4] = {q.x, q.y, q.z, q.w};
-            uint32_t o[4];
-#pragma unroll
-            for (int k = 0; k < 4; ++k) {
-              const float lo = __uint_as_float(u[k] << 16) + elu_from_log2(v[8 * i + 2 * k]);
-              const float hi = __uint_as_float(u[k] & 0xffff0000u) + elu_from_log2(v[8 * i + 2 * k + 1]);
-              o[k] = pack_bf16x2(lo, hi);
-            }
-            pk[i] = make_uint4(o[0], o[1], o[2], o[3]);
-          }
-#pragma unroll
-          for (int i = 0; i < 2; ++i) *reinterpret_cast<uint4*>(arow + ((c0 >> 3) + i) * 2048) = pk[i];
-          if (h & 1) {
-            fence_proxy_async_smem();
-            tc_fence_before_sync();
-            ARRIVE(bar_aready(bar0, h >> 1, RING));
-          }
-          if (ST && !(a.ablate & 2)) {  // the spill goes out after the arrival (see the non-pipelined branch)
-            uint8_t* xo = reinterpret_cast<uint8_t*>(a.X) + tile_image_off((long long)it * ROWS + t, c0 >> 3, 16);
-#pragma unroll
-            for (int i = 0; i < 2; ++i) *reinterpret_cast<uint4*>(xo + i * 2048) = pk[i];
-          }
-        });
-      } else {
-#pragma unroll 1
-      for (int j = 0; j < 2; ++j) {
-        const int cb = 32 * (2 * j + tw);
-        float acc[32];
-        tmem_ld32(tacc + 128 + cb, acc);
-        uint4 px[4];
-#pragma unroll
-        for (int i = 0; i < 4; ++i) px[i] = *reinterpret_cast<const uint4*>(arow + ((cb >> 3) + i) * 2048);
-        tmem_wait_ld();
-        uint4 pk[4];
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-          const uint32_t u[4] = {px[i].x, px[i].y, px[i].z, px[i].w};
+        for (int i = 0; i < 2; ++i) {
+          const uint4 q = *reinterpret_cast<const uint4*>(arow + ((c0 >> 3) + i) * 2048);
+          const uint32_t u[4] = {q.x, q.y, q.z, q.w};
           uint32_t o[4];
 #pragma unroll
           for (int k = 0; k < 4; ++k) {
-            const float lo = __uint_as_float(u[k] << 16) + elu_from_log2(acc[8 * i + 2 * k]);
-            const float hi = __uint_as_float(u[k] & 0xffff0000u) + elu_from_log2(acc[8 * i + 2 * k + 1]);
+            const float lo = __uint_as_float(u[k] << 16) + elu_from_log2(v[8 * i + 2 * k]);
+            const float hi = __uint_as_float(u[k] & 0xffff0000u) + elu_from_log2(v[8 * i + 2 * k + 1]);
             o[k] = pack_bf16x2(lo, hi);
           }
           pk[i] = make_uint4(o[0], o[1], o[2], o[3]);
         }
-        // spilled as a bf16 tile image (fused_engine.cuh) in view-slot row order: the blending head lands it
-        // in its operand tile with one bulk copy per 128 rows.  EA: the global stores are issued AFTER the operand
-        // barrier arrival (fence.proxy.async is a MEMBAR: it would wait for them to be performed first)
-        uint8_t* xo = reinterpret_cast<uint8_t*>(a.X) + tile_image_off((long long)it * ROWS + t, cb >> 3, 16);
-        if (!EA && ST && !(a.ablate & 2)) {
 #pragma unroll
-          for (int i = 0; i < 4; ++i) *reinterpret_cast<uint4*>(xo + i * 2048) = pk[i];
+        for (int i = 0; i < 2; ++i) *reinterpret_cast<uint4*>(arow + ((c0 >> 3) + i) * 2048) = pk[i];
+        if (h & 1) {
+          fence_proxy_async_smem();
+          tc_fence_before_sync();
+          warp_arrive(bar_aready(bar0, h >> 1, kTwinRing));
         }
+        // static net: x is spilled as a bf16 tile image (fused_engine.cuh) in view-slot row order, which the
+        // blending head lands in its operand tile with one bulk copy per 128 rows.  The global stores are issued
+        // AFTER the operand barrier arrival (fence.proxy.async is a MEMBAR: it would wait for them to be performed)
+        if (ST && !(a.ablate & 2)) {
+          uint8_t* xo = reinterpret_cast<uint8_t*>(a.X) + tile_image_off((long long)it * ROWS + t, c0 >> 3, 16);
 #pragma unroll
-        for (int i = 0; i < 4; ++i) *reinterpret_cast<uint4*>(arow + ((cb >> 3) + i) * 2048) = pk[i];
-        fence_proxy_async_smem();
-        tc_fence_before_sync();
-        ARRIVE(bar_aready(bar0, j, RING));
-        if (EA && ST && !(a.ablate & 2)) {
-#pragma unroll
-          for (int i = 0; i < 4; ++i) *reinterpret_cast<uint4*>(xo + i * 2048) = pk[i];
+          for (int i = 0; i < 2; ++i) *reinterpret_cast<uint4*>(xo + i * 2048) = pk[i];
         }
-      }
-
-      }
+      });
 
       TS();  // 14: F6 epilogue done
       if (it + (int)gridDim.x < n_iter) fetch_point(it + (int)gridDim.x);  // next iteration's point
       // ---- F7: vis2 = sigmoid(vis_fc2.2 . ELU(vis1 (vis_fc2.0 x) + b)) * mask ----
-      mbar_wait(bar_acc(bar0, bt, RING), acc_cnt & 1); ++acc_cnt;
+      mbar_wait(acc_full, acc_cnt & 1); ++acc_cnt;
       TS();  // 15: F7 acc ready
       tc_fence_after_sync();
       {
         float part = 0.f;
-        if (EA) {
-          tmem_pipe16<4>(tacc, colh, [&](int h, float* v) {
-            const int c0 = colh(h);
+        tmem_pipe16<4>(tacc, colh, [&](int h, float* v) {
+          const int c0 = colh(h);
 #pragma unroll
-            for (int i = 0; i < 16; ++i)
-              part = fmaf(elu_log2(fmaf(v[i], vis1, cst[T_B7 + c0 + i])), cst[T_W8 + c0 + i], part);
-          });
-        } else {
-#pragma unroll 1
-          for (int j = 0; j < 2; ++j) {
-            const int cb = 32 * (2 * j + tw);
-            float acc[32];
-            tmem_ld32(tacc + cb, acc);
-            tmem_wait_ld();
-#pragma unroll
-            for (int i = 0; i < 32; ++i)
-              part = fmaf(elu_log2(fmaf(acc[i], vis1, cst[T_B7 + cb + i])), cst[T_W8 + cb + i], part);
-          }
-        }
+          for (int i = 0; i < 16; ++i)
+            part = fmaf(elu_log2(fmaf(v[i], vis1, cst[T_B7 + c0 + i])), cst[T_W8 + c0 + i], part);
+        });
         xch7[tw * 128 + t] = part;
       }
       TS();  // 16: F7 partial done
@@ -809,12 +656,11 @@ __global__ void __launch_bounds__(NT * 256 + 64, NT == 1 ? 2 : 1)
       tc_fence_before_sync();
     }
 #undef TS
-#undef ARRIVE
   }
   __syncthreads();
   if (warp == W_ISSUE) {
     tc_fence_after_sync();
-    tmem_dealloc(tmem_base, 256 * NT);
+    tmem_dealloc(tmem_base, 256);
   }
 }
 
@@ -861,12 +707,6 @@ int view_twin3_build(dyn_net* n, const float* P, void* dst_dev, size_t dst_bytes
     add_plan(vis2, 128, 144, m6, 1.f, true, kLog2e, 128, 16, {{{0, 4}}, {{4, 4}, {8, 1}}});
     // vis_fc2.0 on x (vis1 and bias in the epilogue)
     add_plan(vis2_0, 128, 128, identity_map(128, 128), kLog2e, false, -1.f, 0, 0, {{{0, 4}}, {{4, 4}}});
-  };
-  // identity columns 0..K-1 followed by one k-step whose first two columns carry the folded bias (hi, lo)
-  auto bias_map = [](int K) {
-    std::vector<int> m = identity_map(K, K + 16);
-    m[K] = kBiasHi; m[K + 1] = kBiasLo;
-    return m;
   };
   if (n->kind == DYN_NET_STATIC) {
     const StaticLayout& L = n->sl;
@@ -931,7 +771,7 @@ int view_twin3_build(dyn_net* n, const float* P, void* dst_dev, size_t dst_bytes
   return DYN_OK;
 }
 
-int launch_view_twin3(const dyn_net* n, ViewFusedArgs& a, int V, cudaStream_t st, bool elected_arrive) {
+int launch_view_twin3(const dyn_net* n, ViewFusedArgs& a, int V, cudaStream_t st) {
   if (n->twin3.img == nullptr) return fail(DYN_E_INVALID, "net has no twin-warp view images");
   a.wimg = n->twin3.img;
   a.chunks = n->twin3.tab;
@@ -943,11 +783,10 @@ int launch_view_twin3(const dyn_net* n, ViewFusedArgs& a, int V, cudaStream_t st
     int dev = 0;
     DYN_CUDA(cudaGetDevice(&dev));
     DYN_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-#define PREP_VT(VPV, STV) \
-    DYN_CUDA(cudaFuncSetAttribute(view_twin3_kernel<VPV, STV, 1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, twin_smem(1))); \
-    DYN_CUDA(cudaFuncSetAttribute(view_twin3_kernel<VPV, STV, 1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, twin_smem(1)))
-    PREP_VT(8, true); PREP_VT(16, true); PREP_VT(8, false); PREP_VT(16, false);
-#undef PREP_VT
+    DYN_CUDA(cudaFuncSetAttribute(view_twin3_kernel<8, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTwinSmem));
+    DYN_CUDA(cudaFuncSetAttribute(view_twin3_kernel<16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTwinSmem));
+    DYN_CUDA(cudaFuncSetAttribute(view_twin3_kernel<8, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTwinSmem));
+    DYN_CUDA(cudaFuncSetAttribute(view_twin3_kernel<16, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTwinSmem));
     ablate = e ? atoi(e) : 0;
   }
   a.ablate = ablate;
@@ -958,19 +797,13 @@ int launch_view_twin3(const dyn_net* n, ViewFusedArgs& a, int V, cudaStream_t st
   if (grid == 0) return DYN_OK;
   const bool st_net = n->kind == DYN_NET_STATIC;
   ProfScope prof(st_net ? PROF_VIEW_ST : PROF_VIEW_DY, st);
-#define LAUNCH_VT3(VPV, STV)                                                                     \
-  do {                                                                                          \
-    if (elected_arrive) view_twin3_kernel<VPV, STV, 1, true><<<grid, 320, twin_smem(1), st>>>(a);  \
-    else view_twin3_kernel<VPV, STV, 1, false><<<grid, 320, twin_smem(1), st>>>(a);               \
-  } while (0)
   if (st_net) {
-    if (VP == 8) LAUNCH_VT3(8, true);
-    else LAUNCH_VT3(16, true);
+    if (VP == 8) view_twin3_kernel<8, true><<<grid, 320, kTwinSmem, st>>>(a);
+    else view_twin3_kernel<16, true><<<grid, 320, kTwinSmem, st>>>(a);
   } else {
-    if (VP == 8) LAUNCH_VT3(8, false);
-    else LAUNCH_VT3(16, false);
+    if (VP == 8) view_twin3_kernel<8, false><<<grid, 320, kTwinSmem, st>>>(a);
+    else view_twin3_kernel<16, false><<<grid, 320, kTwinSmem, st>>>(a);
   }
-#undef LAUNCH_VT3
   DYN_LAUNCH_CHECK();
   return DYN_OK;
 }

@@ -380,10 +380,11 @@ int dyn_debug_pack_layer(const float* W, const float* bias, int N, int Kw, int N
  * 128-row tile: the layout activations use between the fused kernels. */
 size_t dyn_debug_tile_image_off(long long row, int kgroup, int kgroups);
 
-/* comparison hook: which kernel runs the fused per-view stage: 0 = twin-warp kernel (csrc/view_twin.cu: two
- * independent CTAs per SM), 1 = quad-schedule kernel (csrc/view_quad.cu: one CTA per SM alternating between
- * two tiles), 2 = twin-warp kernel with sub-round pipelined layers (csrc/view_twin3.cu).  The environment
- * variable DYN_VIEW_KERNEL=twin|quad|pipe sets the initial value. */
+/* measurement hook: which kernel runs the fused per-view stage.  -1 (the initial value) = the library's
+ * kernel (csrc/view_twin3.cu).  The comparison variants 0 (round-1 twin-warp kernel), 1 (quad schedule) and
+ * 2 (sub-round pipelined twin kernel without elected arrive) were removed: with any value other than -1 every
+ * fused per-view call (dyn_net_static_fused / dyn_net_dynamic_fused) fails with DYN_E_INVALID and
+ * dyn_last_error() names the variant, so a measurement asking for one cannot time the default instead. */
 void dyn_debug_set_view_kernel(int which);
 
 /* profiling hook: when set, block 0 of the fused static per-view kernel writes clock64()

@@ -1,4 +1,4 @@
-"""Phase timestamps (clock64) of block 0 of the twin-warp static per-view kernel.
+"""Phase timestamps (clock64) of block 0 of the static per-view kernel (csrc/view_twin3.cu).
 
     python profiles/scripts/prof_phases.py > gpurun_out/phases.txt
 """
@@ -19,7 +19,6 @@ NAMES = ["geom+F1 operand", "gather", "wait F1", "F1 epi", "wait F2", "F2 epi+po
 def main():
   DEV = "cuda:0"
   rr.set_precision("bf16")
-  _lib.lib.dyn_debug_set_view_kernel(0)  # twin-warp kernel
   R, S = 8192, 128
   batch, feat_c, feat_f, frame, t, offs = synthetic.make_scene(rays=R, seed=0)
   model, args = synthetic.make_model(64, 64)

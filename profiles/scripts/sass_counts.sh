@@ -12,7 +12,7 @@ echo "as a substring of \`UTCHMMA\`; no \`UTMALDG\` (the bulk copies are 1-D: we
 echo
 echo "| object | UTCHMMA | LDTM | STTM | UBLKCP | UTMALDG | SYNCS | MUFU.EX2 | legacy HMMA |"
 echo "|---|---|---|---|---|---|---|---|---|"
-for f in view_twin3 view_twin view_quad chains_twin chains_fused attention_tc linear_tc train_tc; do
+for f in view_twin3 chains_twin chains_fused attention_tc linear_tc train_tc; do
   cuobjdump -sass $f.o > /tmp/_sass_$f.txt 2>/dev/null
   c() { grep -c "$1" /tmp/_sass_$f.txt; }
   legacy=$(grep "HMMA" /tmp/_sass_$f.txt | grep -vc "UTCHMMA")
