@@ -25,6 +25,27 @@ NET_DYNAMIC, NET_STATIC, NET_MOTION = 0, 1, 2
 
 _vp, _i, _f, _sz = C.c_void_p, C.c_int, C.c_float, C.c_size_t
 
+# struct dyn_objective_in / dyn_objective_grad (pointer fields, in header order)
+OBJ_IN_FIELDS = ("rgb", "rgb_dy", "rgb_static", "depth", "mask", "weights", "weights_dy", "weights_st", "s_vals",
+                 "render_flows", "ref_dy_rgb", "ref_dy_mask", "a_rgb", "a_mask", "a_occ_map", "occ_weights",
+                 "pts_traj_ref", "pts_traj_anchor", "sf_seq", "a_dy_rgb", "a_dy_mask", "a_dy_occ_map", "st_rgb",
+                 "gt_rgb", "disp", "motion_mask", "static_mask", "flows", "flow_masks", "dist_mid", "dist_interval")
+OBJ_GRAD_FIELDS = ("rgb", "rgb_dy", "rgb_static", "depth", "weights", "weights_dy", "weights_st", "render_flows",
+                   "ref_dy_rgb", "a_rgb", "pts_traj_ref", "pts_traj_anchor", "sf_seq", "a_dy_rgb", "st_rgb")
+
+
+class ObjectiveIn(C.Structure):
+  _fields_ = [(n, _i) for n in ("R", "S", "K", "T", "F")] + [(n, _vp) for n in OBJ_IN_FIELDS]
+
+
+class ObjectiveGrad(C.Structure):
+  _fields_ = [(n, _vp) for n in OBJ_GRAD_FIELDS]
+
+
+OBJ_NSUMS, OBJ_NTERMS, OBJ_NCOEF = 32, 8, 7
+(OBJ_RGB, OBJ_TEMPORAL, OBJ_DYREGION, OBJ_DYNAMIC, OBJ_DISP, OBJ_FLOW, OBJ_CYCLE, OBJ_REG, OBJ_ENTROPY,
+ OBJ_DISTORTION, OBJ_STATIC, OBJ_STATIC_EXTRA, OBJ_BOOTSTRAP) = (1 << i for i in range(13))
+
 # name -> (restype, argtypes); mirrors include/dynibar_b200.h one to one
 SIGNATURES = {
     "dyn_version": (_i, []),
@@ -100,6 +121,10 @@ SIGNATURES = {
     "dyn_encoder_backward": (_i, [_vp, _sz, _vp, _i, _i, _i, _vp, _vp, _vp, _sz, _vp, _sz, _vp, _i, _vp]),
     "dyn_flow_sceneflow": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i,
                                 _vp, _vp, _vp]),
+    "dyn_objective_workspace_bytes": (_sz, [_i]),
+    "dyn_objective_sums": (_i, [C.POINTER(ObjectiveIn), _i, _vp, _vp, _sz, _vp]),
+    "dyn_objective_finalize": (_i, [_vp, _i, C.POINTER(C.c_double), _vp, _vp, _vp, _vp]),
+    "dyn_objective_backward": (_i, [C.POINTER(ObjectiveIn), _i, _vp, _vp, _vp, C.POINTER(ObjectiveGrad), _vp]),
 }
 
 for _name, (_res, _args) in SIGNATURES.items():

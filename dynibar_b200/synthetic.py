@@ -126,6 +126,25 @@ def make_scene(H=288, W=512, V_dy=8, V_st=8, C=32, num_frames=24, frame_idx=10,
   return batch, feat_c, feat_f, frame, t, offs
 
 
+def make_supervision(batch, n_flow=6, seed=0):
+  """`batch` plus seeded per-ray supervision in the layout RaySamplerSingleImage.random_sample returns
+  (sample_ray.py:262-331): rgb [R,3] in [0,1), disp [R], binary motion_mask / static_mask [R], flows [n_flow,R,2]
+  and binary masks [n_flow,R,1], on the device of batch['ray_o']."""
+  R = batch["ray_o"].shape[0]
+  g = torch.Generator().manual_seed(seed)
+  sup = {
+      "rgb": torch.rand(R, 3, generator=g),
+      "disp": torch.rand(R, generator=g) * 0.9 + 0.05,
+      "motion_mask": (torch.rand(R, generator=g) > 0.5).float(),
+      "static_mask": (torch.rand(R, generator=g) > 0.6).float(),
+      "flows": torch.randn(n_flow, R, 2, generator=g) * 2.0,
+      "masks": (torch.rand(n_flow, R, 1, generator=g) > 0.3).float(),
+  }
+  out = dict(batch)
+  out.update(to_device(sup, batch["ray_o"].device))
+  return out
+
+
 def make_model(N_samples=64, N_importance=64, num_frames=24, args=None, seed=0,
                mono=False, sigma_bias=-4.0, coeff_std=1e-2):
   """Duck-typed model namespace with the attributes render_rays_* read

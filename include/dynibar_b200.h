@@ -331,6 +331,79 @@ int dyn_traj_combine_backward(const float* g_out, const float* D, int n, int nb,
 int dyn_flow_backward(const float* weights, const float* pts_seq, const float* src_cams, const float* g_flows,
                       int n_flow, int R, int S, float* g_weights, float* g_pts_seq, void* stream);
 
+/* ---- training objective: train.py:300-458 (the loss of one training step), the static-bootstrap loss of
+ * train.py:187-196 and eff_distloss_native (mip-NeRF 360 distortion, prefix-sum form), with the criteria of
+ * ibrnet/criterion.py.  One warp per ray; every per-ray quantity is evaluated in fp64.
+ *
+ * `in` describes the tensors (all [R]-leading rows dense fp32; masks as 0/1 floats):
+ *   outputs_coarse_ref      rgb, rgb_dy, rgb_static [R,3]; depth, mask [R]; weights, weights_dy, weights_st,
+ *                           s_vals [R,S]; render_flows [F,R,2]
+ *   outputs_coarse_ref_dy   ref_dy_rgb [R,3], ref_dy_mask [R]
+ *   outputs_coarse_anchor   a_rgb [R,3], a_mask, a_occ_map [R], occ_weights [R,S],
+ *                           pts_traj_ref, pts_traj_anchor [K,R,S,3], sf_seq [T,R,S,3]
+ *   outputs_coarse_anchor_dy a_dy_rgb [R,3], a_dy_mask, a_dy_occ_map [R]
+ *   outputs_coarse_st       st_rgb [R,3]
+ *   ray_batch               gt_rgb [R,3], disp, motion_mask, static_mask [R], flows [F,R,2], flow_masks [F,R,1]
+ *   eff_distloss_native     dist_mid, dist_interval [R,S] with weights [R,S] = w; when both are NULL the
+ *                           distortion term reads weights[:, :S-1], mid(s_vals) and diff(s_vals) instead.
+ * Only the tensors of the enabled `terms` (DYN_OBJ_* bits) are read; the others may be NULL.
+ *
+ * dyn_objective_sums writes the DYN_OBJ_NSUMS fp64 sums of the batch (numerators, denominators and the ray /
+ * element counts of the means; slots DYN_OBJ_SUM_*), reduced per block in warp order and across blocks in block
+ * order: no float atomics, bit-identical between runs.  Sums of disjoint ray batches add up to the sums of their
+ * union, so sharded callers all-reduce this vector (SUM) before dyn_objective_finalize.
+ * dyn_objective_finalize turns a sums vector into loss [1] and the DYN_OBJ_NTERMS term values (fp32; order
+ * rgb, flow, disp, distortion, entropy, static, cycle, reg) and `scales` [DYN_OBJ_NSUMS] fp64: d loss / d each
+ * numerator.  coef_host [DYN_OBJ_NCOEF] (HOST): dynamic-rgb factor 1/10^divisor, disp, flow, cycle, reg,
+ * entropy and distortion weights.
+ * dyn_objective_backward writes every non-NULL gradient of `grad` in full from the upstream gradients g_loss [1]
+ * and g_terms [DYN_OBJ_NTERMS] (device; either may be NULL = 0) and the scales of the finalize step.
+ * One launch each; nothing synchronises. */
+#define DYN_OBJ_RGB 0x001            /* Charbonnier of ref.rgb under ref.mask (train.py:304) */
+#define DYN_OBJ_TEMPORAL 0x002       /* temporal Charbonnier of anchor.rgb (:305-307) */
+#define DYN_OBJ_DYREGION 0x004       /* Charbonnier of ref.rgb_dy under mask * motion_mask (:309-316) */
+#define DYN_OBJ_DYNAMIC 0x008        /* ref_dy.rgb and anchor_dy.rgb under motion_mask, / 10^divisor (:318-329) */
+#define DYN_OBJ_DISP 0x010           /* disparity L1 (:330-343) */
+#define DYN_OBJ_FLOW 0x020           /* flow L1 (:344-352) */
+#define DYN_OBJ_CYCLE 0x040          /* trajectory cycle L1 (:353-371) */
+#define DYN_OBJ_REG 0x080            /* scene-flow regularisers (:373-397) */
+#define DYN_OBJ_ENTROPY 0x100        /* weight-ratio entropy (:399-413) */
+#define DYN_OBJ_DISTORTION 0x200     /* eff_distloss_native (:415-423) */
+#define DYN_OBJ_STATIC 0x400         /* static Charbonnier of ref.rgb_static (:425-435) */
+#define DYN_OBJ_STATIC_EXTRA 0x800   /* divisor > 4: zero dynamic weight where ratio < 0.1 (:437-445) */
+#define DYN_OBJ_BOOTSTRAP 0x1000     /* static bootstrap, Charbonnier of st.rgb (:187-196) */
+#define DYN_OBJ_NSUMS 32
+#define DYN_OBJ_NTERMS 8
+#define DYN_OBJ_NCOEF 7
+
+typedef struct dyn_objective_in {
+  int R, S, K, T, F; /* rays, samples, trajectory views, sf_seq steps, flow views */
+  const float *rgb, *rgb_dy, *rgb_static, *depth, *mask, *weights, *weights_dy, *weights_st, *s_vals,
+      *render_flows;
+  const float *ref_dy_rgb, *ref_dy_mask;
+  const float *a_rgb, *a_mask, *a_occ_map, *occ_weights, *pts_traj_ref, *pts_traj_anchor, *sf_seq;
+  const float *a_dy_rgb, *a_dy_mask, *a_dy_occ_map;
+  const float* st_rgb;
+  const float *gt_rgb, *disp, *motion_mask, *static_mask, *flows, *flow_masks;
+  const float *dist_mid, *dist_interval;
+} dyn_objective_in;
+
+typedef struct dyn_objective_grad { /* same shapes as the inputs of the same names */
+  float *rgb, *rgb_dy, *rgb_static, *depth, *weights, *weights_dy, *weights_st, *render_flows;
+  float* ref_dy_rgb;
+  float *a_rgb, *pts_traj_ref, *pts_traj_anchor, *sf_seq;
+  float* a_dy_rgb;
+  float* st_rgb;
+} dyn_objective_grad;
+
+size_t dyn_objective_workspace_bytes(int R);
+int dyn_objective_sums(const dyn_objective_in* in, int terms, double* sums, void* workspace,
+                       size_t workspace_bytes, void* stream);
+int dyn_objective_finalize(const double* sums, int terms, const double* coef_host, float* loss, float* term_values,
+                           double* scales, void* stream);
+int dyn_objective_backward(const dyn_objective_in* in, int terms, const double* scales, const float* g_loss,
+                           const float* g_terms, const dyn_objective_grad* grad, void* stream);
+
 /* Unit-test hooks of the tensor-core training products (csrc/train_tc.cu; bf16 operands, fp32 accumulation):
  * dyn_debug_tc_grad_w: dW[out,width] += dz[rows,out]^T (x[rows,width] * kscale[rows] or 1); out, width <= 256.
  * dyn_debug_tc_grad_in: din[rows,width] = dz[rows,out] W[out, 0:width] (W row-major with ldw columns). */
