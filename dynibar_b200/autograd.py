@@ -15,6 +15,7 @@ of the path, so that `render_ray.render_rays_mono(..., is_train=True)` is differ
                         :423-527) incl. the ray transformer: gradients w.r.t. every parameter, the gathered
                         rgb_feat and (dynamic) the sample points (csrc/nets_train.cu, fp32).
   * `composite_vanilla` raw2outputs_vanilla (render_ray.py:134-211).
+                        The two compositors are also the evaluation path's: under no_grad only their forward runs.
   * `traj_combine`      compute_traj_pts and the displacements built from it (render_ray.py:361-369, :462-500).
   * `optical_flow`      compute_optical_flow (render_ray.py:333-358).
 
@@ -38,9 +39,10 @@ class _Composite(torch.autograd.Function):
     rays = torch.empty(R, 11, device=dev)
     samp = torch.empty(5, R, S, device=dev)
     rd, rs, zz = f32c(raw_dy), f32c(raw_st), f32c(z_vals)
+    A = Args()
     with torch.cuda.device(dev):
-      check(lib.dyn_composite(ptr(rd), ptr(rs), ptr(zz), ptr(f32c(mask_dy)), V_dy, int(min_dy),
-                              ptr(f32c(mask_st)), V_st, int(min_st), R, S, ptr(rays), ptr(samp), stream()))
+      check(lib.dyn_composite(ptr(rd), ptr(rs), ptr(zz), A(mask_dy), V_dy, int(min_dy), A(mask_st), V_st, int(min_st),
+                              R, S, ptr(rays), ptr(samp), stream()))
     ctx.save_for_backward(rd, rs, zz)
     ctx.mark_non_differentiable(rays[:, 10])
     return rays, samp
@@ -59,7 +61,8 @@ class _Composite(torch.autograd.Function):
 
 
 def composite(raw_dy, raw_st, z_vals, mask_dy, mask_st, min_views_dy=1, min_views_st=1):
-  """Differentiable raw2outputs: same 11-key dict as render_ray._composite."""
+  """raw2outputs, differentiable w.r.t. raw_dy / raw_st -> the reference's 11-key dict.  mask_* [R,S,V(,1)]: a
+  sample counts when more than min_views_* of its V views see it."""
   rays, samp = _Composite.apply(raw_dy, raw_st, z_vals, mask_dy, mask_st, min_views_dy, min_views_st)
   return OrderedDict([
       ("rgb", rays[:, 0:3]), ("rgb_static", rays[:, 3:6]), ("rgb_dy", rays[:, 6:9]),
@@ -137,32 +140,22 @@ class _MotionMLP(torch.autograd.Function):
     with torch.cuda.device(x.device):
       check(lib.dyn_motion_mlp_backward(net.handle, ptr(x), ptr(gc), N, ctx.ws.data_ptr(), ctx.nbytes,
                                         ptr(d_params), ptr(d_x) if d_x is not None else None, ctx.prec, stream()))
-    grads, o = [], 0
-    for shp in ctx.shapes:  # state_dict order == parameters() order == the blob's order (weights.py)
-      n = 1
-      for d in shp:
-        n *= d
-      grads.append(d_params[o:o + n].reshape(shp))
-      o += n
-    return (d_x.reshape(ctx.in_shape) if d_x is not None else None, None, None) + tuple(grads)
+    return ((d_x.reshape(ctx.in_shape) if d_x is not None else None, None, None)
+            + tuple(_split_param_grads(d_params, ctx.shapes)))
 
 
 def _prec_code(precision):
   """None -> the library-wide setting of render_ray (`set_precision` / `precision_scope`)."""
-  from dynibar_b200 import render_ray, _lib
-  if precision is None:
-    return render_ray._prec()
-  return {"fp32": _lib.PREC_FP32, "bf16": _lib.PREC_BF16}[precision]
+  from dynibar_b200 import render_ray
+  return render_ray._prec() if precision is None else render_ray._PREC[precision]
 
 
 def motion_mlp(module, xyzt, precision=None):
   """Differentiable MotionMLP.forward on [...,4] rows; honours `sf_mag_div` like render_ray.motion_mlp_forward.
   precision "bf16": the products run on tcgen05 (bf16 operands, fp32 accumulation / master weights)."""
-  from dynibar_b200 import weights
-  m = weights.de_parallel(module)
-  out = _MotionMLP.apply(xyzt, module, _prec_code(precision), *m.parameters())
-  div = float(getattr(m, "sf_mag_div", 1.0))
-  return out / div if div != 1.0 else out
+  from dynibar_b200 import render_ray, weights
+  out = _MotionMLP.apply(xyzt, module, _prec_code(precision), *weights.de_parallel(module).parameters())
+  return render_ray._sf_mag_div(module, out)
 
 
 def _split_param_grads(d_params, shapes):
@@ -302,7 +295,7 @@ class _CompositeVanilla(torch.autograd.Function):
 
 
 def composite_vanilla(raw, z_vals, mask, min_views=1):
-  """Differentiable raw2outputs_vanilla: same 6-key dict as render_ray._composite_vanilla."""
+  """raw2outputs_vanilla, differentiable w.r.t. raw -> the reference's 6-key dict (mask: see composite)."""
   rays, samp = _CompositeVanilla.apply(raw, z_vals, mask, min_views)
   return OrderedDict([
       ("rgb", rays[:, 0:3]), ("depth", rays[:, 3]), ("weights", samp[0]),

@@ -7,12 +7,14 @@ reference): `render_rays_mv` (render_ray.py:600), `render_rays_mono` (:870),
 `compute_src_plucker_coordinate` (:380), `z_to_s` (:399).
 
 All math runs in `csrc/` kernels through the C ABI (include/dynibar_b200.h);
-this file only allocates tensors and sequences calls.  `render_rays_mono` is
-differentiable (training, SURVEY 8(f) f2): when gradients are enabled and the
-model's parameters or the feature maps require grad it runs the training
-path (`_render_mono_train`, autograd Functions of dynibar_b200/autograd.py over
-the backward kernels).  `render_rays_mv` is the evaluation path (the reference
-calls it under no_grad) and refuses inputs that require grad.
+this file only allocates tensors and sequences calls.  `_render_pass` (one pass
+at the reference time) and `_cross_time` (the anchor branch) state that sequence
+once.  `render_rays_mono` is differentiable (training, SURVEY 8(f) f2): when
+gradients are enabled and the model's parameters or the feature maps require
+grad it runs the same sequence with `train=True`, and the stages whose kernels
+differ use the autograd Functions of dynibar_b200/autograd.py over the backward
+kernels.  `render_rays_mv` is the evaluation path (the reference calls it under
+no_grad) and refuses inputs that require grad.
 """
 
 from collections import OrderedDict
@@ -25,6 +27,7 @@ import weakref
 import torch
 
 from dynibar_b200 import _lib
+from dynibar_b200 import autograd as ag
 from dynibar_b200 import weights as _weights
 from dynibar_b200._lib import lib, ptr, f32c, check, stream, dev_of, Args
 from dynibar_b200.projection import project_gather
@@ -37,8 +40,6 @@ from dynibar_b200.projection import project_gather
 _PREC = {"fp32": _lib.PREC_FP32, "bf16": _lib.PREC_BF16}
 PRECISION = _PREC[os.environ.get("DYNIBAR_B200_PRECISION", "bf16")]
 _tls = threading.local()
-# DYN_PREC_BF16: use the fused per-view kernels (False = staged tensor-core layers)
-USE_FUSED = True
 
 
 def set_precision(name):
@@ -160,10 +161,7 @@ def motion_mlp_forward(module, xyzt):
   with torch.cuda.device(dev):
     check(lib.dyn_motion_mlp(net.handle, ptr(x), N, ptr(out), ws.data_ptr(), nbytes, _prec(),
                              stream()))
-  div = float(getattr(_weights.de_parallel(module), "sf_mag_div", 1.0))
-  if div != 1.0:
-    out = out / div
-  return out.reshape(xyzt.shape[:-1] + (out.shape[-1],))
+  return _sf_mag_div(module, out).reshape(xyzt.shape[:-1] + (out.shape[-1],))
 
 
 def motion_coefficients(module, pts, t):
@@ -178,10 +176,13 @@ def motion_coefficients(module, pts, t):
   with torch.cuda.device(dev):
     check(lib.dyn_motion_coeffs(net.handle, A(pts), float(t), R, S, ptr(out),
                                 ws.data_ptr(), nbytes, _prec(), stream()))
+  return _sf_mag_div(module, out)
+
+
+def _sf_mag_div(module, out):
+  """MotionMLP.forward divides its output by the module's sf_mag_div (mlp_network.py:617)."""
   div = float(getattr(_weights.de_parallel(module), "sf_mag_div", 1.0))
-  if div != 1.0:  # MotionMLP.forward divides its output (mlp_network.py:617)
-    out = out / div
-  return out
+  return out / div if div != 1.0 else out
 
 
 def displaced_points(pts, coeff, basis, frame_idx, offsets, num_vv=0):
@@ -401,47 +402,14 @@ def net_dynamic_fused(module, pts, pts_seq, ray_dir, query_cam, src_rgbs, src_ca
 # ---------------------------------------------------------------------------
 # a12
 # ---------------------------------------------------------------------------
-def _composite(raw_dy, raw_st, z, mask_dy, V_dy, min_dy, mask_st, V_st, min_st):
-  R, S = z.shape
-  dev = dev_of(z)
-  rays = torch.empty(R, 11, device=dev)
-  samp = torch.empty(5, R, S, device=dev)
-  A = Args()
-  with torch.cuda.device(dev):
-    check(lib.dyn_composite(A(raw_dy), A(raw_st), A(z), A(mask_dy),
-                            V_dy, min_dy, A(mask_st), V_st, min_st, R, S, ptr(rays),
-                            ptr(samp), stream()))
-  return OrderedDict([
-      ("rgb", rays[:, 0:3]), ("rgb_static", rays[:, 3:6]), ("rgb_dy", rays[:, 6:9]),
-      ("depth", rays[:, 9]), ("alpha_dy", samp[0]), ("weights_dy", samp[1]),
-      ("weights_st", samp[2]), ("alpha", samp[3]), ("weights", samp[4]),
-      ("mask", rays[:, 10] > 0.5), ("z_vals", z),
-  ])
-
-
-def _composite_vanilla(raw, z, mask, V, min_views):
-  R, S = z.shape
-  dev = dev_of(z)
-  rays = torch.empty(R, 5, device=dev)
-  samp = torch.empty(2, R, S, device=dev)
-  A = Args()
-  with torch.cuda.device(dev):
-    check(lib.dyn_composite_vanilla(A(raw), A(z), A(mask), V, min_views,
-                                    R, S, ptr(rays), ptr(samp), stream()))
-  return OrderedDict([
-      ("rgb", rays[:, 0:3]), ("depth", rays[:, 3]), ("weights", samp[0]),
-      ("mask", rays[:, 4] > 0.5), ("alpha", samp[1]), ("z_vals", z),
-  ])
-
-
 def raw2outputs(raw_dy, raw_static, z_vals, mask_dy, mask_static, raw_noise_std=0.0):
   """render_ray.py:214-330; mask_* are the per-sample [R,S] validity masks."""
-  return _composite(raw_dy, raw_static, z_vals, mask_dy.float(), 1, 0, mask_static.float(), 1, 0)
+  return ag.composite(raw_dy, raw_static, z_vals, mask_dy.float()[..., None], mask_static.float()[..., None], 0, 0)
 
 
 def raw2outputs_vanilla(raw, z_vals, mask):
   """render_ray.py:134-211."""
-  return _composite_vanilla(raw, z_vals, mask.float(), 1, 0)
+  return ag.composite_vanilla(raw, z_vals, mask.float()[..., None], 0)
 
 
 # ---------------------------------------------------------------------------
@@ -514,50 +482,95 @@ def _with_host_copies(ray_batch, model, basis_names):
   return rb, basis
 
 
-def _render_pass(ray_batch, feat_dy, feat_st, pts, z, s, t, frame_idx, offsets, num_vv, net_dy,
-                 net_st, motion, basis, flow_views, sf_k, want_extras=True, want_vanilla_st=False,
-                 want_aux=False):
-  """One coarse-or-fine evaluation at the reference time
-  (render_ray.py:455-597 == :672-782 == :951-1096)."""
+# The stages of the sequence whose kernels differ between evaluation and training (`train`): the forward-only
+# kernels, or the autograd Functions of dynibar_b200/autograd.py over the forward/backward kernels.
+def _coefficients(train, motion, pts, t):
+  """Motion coefficients [R,S,3*nb] at time t with the last round(0.1*S) samples zeroed (render_ray.py:957-958,
+  :1126-1127)."""
+  if not train:
+    return motion_coefficients(motion, pts, t)
+  R, S = pts.shape[:2]
+  keep = torch.ones(1, S, 1, device=pts.device)
+  keep[:, -int(round(S * 0.1)):] = 0.0  # the reference's x[:, -n:]: n == 0 (S <= 5) zeroes every sample
+  xyzt = torch.cat([pts, torch.full((R, S, 1), t, device=pts.device)], dim=-1)
+  return ag.motion_mlp(motion, xyzt) * keep
+
+
+def _basis_rows(basis, pairs, dev):
+  """D[i] = basis[a_i] - basis[b_i] ((None, None): a zero row) on the device; the host basis [T, nb] is indexed like
+  the reference's (negative indices wrap)."""
+  zero = torch.zeros_like(basis[0])
+  return torch.stack([basis[a] - basis[b] if a is not None else zero for a, b in pairs]).to(dev)
+
+
+def _displace(train, pts, coeff, basis, frame_idx, offsets, num_vv=0):
+  """pts + traj(frame_idx + o) - traj(frame_idx) per offset, then num_vv copies of pts -> [n+num_vv,R,S,3]."""
+  if not train:
+    return displaced_points(pts, coeff, basis, frame_idx, offsets, num_vv)
+  pairs = [(frame_idx + o, frame_idx) for o in offsets] + [(None, None)] * num_vv
+  return ag.traj_combine(coeff, _basis_rows(basis, pairs, pts.device), pts)
+
+
+def _deltas(train, coeff, basis, frames_a, frames_b):
+  """traj(frames_a[i]) - traj(frames_b[i]) -> [n,R,S,3]."""
+  if not train:
+    return traj_deltas(coeff, basis, frames_a, frames_b)
+  return ag.traj_combine(coeff, _basis_rows(basis, list(zip(frames_a, frames_b)), coeff.device))
+
+
+def _fused(train, *cameras):
+  """Evaluation in bf16 mode with at most 16 views per branch runs gather + per-view MLP chain + pooling as one
+  tcgen05 kernel per branch: the [R,S,V,35] gather output and the per-view activations never reach HBM.  Otherwise
+  the gather, then the networks' layers."""
+  return not train and _prec() == _lib.PREC_BF16 and all(c.shape[1] <= 16 for c in cameras)
+
+
+def _dynamic_branch(train, fused, net, pts, pts_net, seq, ray_dir, cam, rgbs, cams, feat, t):
+  """DynibarDynamic on the views `cams` seen from the displaced points `seq` -> raw [R,S,4], mask [R,S,V,1].  As in
+  the reference the gather takes the reference-time points `pts` and the network `pts_net` (:1178-1196)."""
+  if fused:
+    return net_dynamic_fused(net, pts_net, seq, ray_dir, cam, rgbs, cams, featmaps_channels_last(feat), t)
+  gather, net_fn = (ag.project_gather, ag.net_dynamic) if train else (project_gather, net_dynamic_forward)
+  f, _, m = gather(pts, seq, cam, rgbs, cams, feat)
+  return net_fn(net, pts_net, f, ray_dir, m, t), m
+
+
+def _render_pass(ray_batch, feat_dy, feat_st, pts, z, s, t, frame_idx, offsets, num_vv, net_dy, net_st, motion,
+                 basis, flow_views, sf_k, train=False, want_extras=True, want_vanilla_st=False):
+  """One coarse-or-fine evaluation at the reference time (render_ray.py:455-597 == :672-782 == :951-1096)
+  -> the composited dicts (joint, dynamic, static or None) and what the cross-time branch reuses."""
   cam, ray_o, ray_d = ray_batch["camera"], ray_batch["ray_o"], ray_batch["ray_d"]
+  cams_dy, cams_st = ray_batch["src_cameras"], ray_batch["static_src_cameras"]
   ref_plucker = compute_ref_plucker_coordinate(ray_o, ray_d)  # [d_hat, o x d_hat]
   ray_dir = ref_plucker[:, :3]  # == F.normalize(ray_d) (render_ray.py:455)
-  coeff = motion_coefficients(motion, pts, t)
-  seq = displaced_points(pts, coeff, basis, frame_idx, offsets, num_vv)
-  fused = (_prec() == _lib.PREC_BF16 and USE_FUSED and ray_batch["src_cameras"].shape[1] <= 16
-           and ray_batch["static_src_cameras"].shape[1] <= 16)
+  coeff = _coefficients(train, motion, pts, t)
+  seq = _displace(train, pts, coeff, basis, frame_idx, offsets, num_vv)
+  fused = _fused(train, cams_dy, cams_st)
+  raw_dy, m_dy = _dynamic_branch(train, fused, net_dy, pts, pts, seq, ray_dir, cam, ray_batch["src_rgbs"], cams_dy,
+                                 feat_dy, t)
   if fused:
-    # gather + per-view MLP chain + pooling in one tcgen05 kernel per branch: the
-    # [R,S,V,35] gather output and the per-view activations never reach HBM
-    raw_dy, m_dy = net_dynamic_fused(net_dy, pts, seq, ray_dir, cam, ray_batch["src_rgbs"],
-                                     ray_batch["src_cameras"], featmaps_channels_last(feat_dy), t)
-    raw_st, m_st = net_static_fused(net_st, pts, ray_o, ray_d, cam, ray_batch["static_src_rgbs"],
-                                    ray_batch["static_src_cameras"],
+    raw_st, m_st = net_static_fused(net_st, pts, ray_o, ray_d, cam, ray_batch["static_src_rgbs"], cams_st,
                                     featmaps_channels_last(feat_st))
   else:
-    f_dy, _, m_dy = project_gather(pts, seq, cam, ray_batch["src_rgbs"], ray_batch["src_cameras"],
-                                   feat_dy)
-    f_st, rd_st, m_st = project_gather(pts, None, cam, ray_batch["static_src_rgbs"],
-                                       ray_batch["static_src_cameras"], feat_st)
-    raw_dy = net_dynamic_forward(net_dy, pts, f_dy, ray_dir, m_dy, t)
-    raw_st = net_static_forward(net_st, pts, ref_plucker,
-                                compute_src_plucker_coordinate(pts, ray_batch["static_src_cameras"]),
-                                f_st, rd_st, m_st)
-  V_dy, V_st = m_dy.shape[2], m_st.shape[2]
+    gather, net_fn = (ag.project_gather, ag.net_static) if train else (project_gather, net_static_forward)
+    f_st, rd_st, m_st = gather(pts, None, cam, ray_batch["static_src_rgbs"], cams_st, feat_st)
+    raw_st = net_fn(net_st, pts, ref_plucker, compute_src_plucker_coordinate(pts, cams_st), f_st, rd_st, m_st)
   # a sample counts when MORE THAN ONE view sees it (render_ray.py:524-529)
-  out = _composite(raw_dy, raw_st, z, m_dy, V_dy, 1, m_st, V_st, 1)
-  out_dy = _composite_vanilla(raw_dy, z, m_dy, V_dy, 1)
-  out_st = _composite_vanilla(raw_st, z, m_st, V_st, 1) if want_vanilla_st else None
+  out = ag.composite(raw_dy, raw_st, z, m_dy, m_st, 1, 1)
+  out_dy = ag.composite_vanilla(raw_dy, z, m_dy, 1)
+  out_st = ag.composite_vanilla(raw_st, z, m_st, 1) if want_vanilla_st else None
   if want_extras:
     nflow = seq.shape[0] if flow_views is None else flow_views
-    flows, exp_sf = _flow_sceneflow(out["weights"], seq, ray_batch["src_cameras"],
-                                    ray_batch["uv_grid"], coeff, basis, frame_idx, sf_k, nflow)
+    uv = ray_batch["uv_grid"]
+    if train:  # exp_sf is detached in the reference (:1086-1096)
+      flows = ag.optical_flow(out["weights"], seq[:nflow], cams_dy[:, :nflow], uv)
+      _, exp_sf = _flow_sceneflow(out["weights"], seq, cams_dy, uv, coeff, basis, frame_idx, sf_k, 1)
+    else:
+      flows, exp_sf = _flow_sceneflow(out["weights"], seq, cams_dy, uv, coeff, basis, frame_idx, sf_k, nflow)
     out["render_flows"] = flows
     out["s_vals"] = s
     out["exp_sf"] = exp_sf
-  if want_aux:
-    return out, out_dy, out_st, dict(coeff=coeff, raw_st=raw_st, m_st=m_st, ray_dir=ray_dir)
-  return out, out_dy, out_st
+  return out, out_dy, out_st, dict(coeff=coeff, raw_st=raw_st, m_st=m_st, ray_dir=ray_dir)
 
 
 def render_rays_mv(frame_idx, time_embedding, time_offset, ray_batch, model, projector,
@@ -579,16 +592,16 @@ def render_rays_mv(frame_idx, time_embedding, time_offset, ray_batch, model, pro
     ray_batch, hb = _with_host_copies(ray_batch, model, ("trajectory_basis", "trajectory_basis_fine"))
     pts, z, _ = sample_along_camera_ray(ray_batch["ray_o"], ray_batch["ray_d"],
                                         ray_batch["depth_range"], N_samples, inv_uniform, det, jitter)
-    out_c, _, _ = _render_pass(ray_batch, coarse_featmaps[0], coarse_featmaps[2], pts, z, None, t,
-                               fidx, offs, 0, model.net_coarse_dy, model.net_coarse_st,
-                               model.motion_mlp, hb["trajectory_basis"], None, 2, want_extras=False)
+    out_c = _render_pass(ray_batch, coarse_featmaps[0], coarse_featmaps[2], pts, z, None, t, fidx, offs, 0,
+                         model.net_coarse_dy, model.net_coarse_st, model.motion_mlp, hb["trajectory_basis"], None,
+                         2, want_extras=False)[0]
     ret["outputs_coarse_ref"] = out_c
     zf = resample_depths(z, out_c["weights"], N_importance, inv_uniform, det, u)
     pts_f, s = points_from_depths(ray_batch["ray_o"], ray_batch["ray_d"], zf,
                                   ray_batch["depth_range"])
-    out_f, out_f_dy, _ = _render_pass(ray_batch, fine_featmaps[0], fine_featmaps[2], pts_f, zf, s,
-                                      t, fidx, offs, 0, model.net_fine_dy, model.net_fine_st,
-                                      model.motion_mlp_fine, hb["trajectory_basis_fine"], None, 2)
+    out_f, out_f_dy = _render_pass(ray_batch, fine_featmaps[0], fine_featmaps[2], pts_f, zf, s, t, fidx, offs, 0,
+                                   model.net_fine_dy, model.net_fine_st, model.motion_mlp_fine,
+                                   hb["trajectory_basis_fine"], None, 2)[:2]
     ret["outputs_fine_ref"] = out_f
     ret["outputs_fine_ref_dy"] = out_f_dy
     ret["outputs_fine_anchor"] = None
@@ -601,59 +614,63 @@ def render_rays_mono(frame_idx, time_embedding, time_offset, ray_batch, model, f
                      det=False, white_bkgd=False, is_train=True, num_vv=2, jitter=None, precision=None):
   """Coarse-only rendering for monocular video (render_ray.py:870-1277), including the
   cross-time branch (:1099-1270) when is_train=True.  With gradients enabled and parameters / feature
-  maps that require grad the differentiable fp32 training path runs (`_render_mono_train`); otherwise
-  the forward-only kernels (fused tcgen05 path in bf16 mode) under no_grad."""
-  if _wants_grad(model, featmaps):
-    with precision_scope(precision):
+  maps that require grad it is differentiable (training, see _render_mono); otherwise the forward-only kernels
+  (fused tcgen05 path in bf16 mode) run under no_grad."""
+  with precision_scope(precision):
+    if _wants_grad(model, featmaps):
       return _render_mono_train_chunked(frame_idx, time_embedding, time_offset, ray_batch, model, featmaps,
                                         N_samples, args, inv_uniform, det, is_train, num_vv, jitter)
-  with torch.no_grad(), precision_scope(precision):
-    t = _scalar(time_embedding[0].float())
-    ray_batch, hb = _with_host_copies(ray_batch, model, ("trajectory_basis",))
-    basis = hb["trajectory_basis"]
-    fidx = int(frame_idx[0])
-    pts, z, s = sample_along_camera_ray(ray_batch["ray_o"], ray_batch["ray_d"],
-                                        ray_batch["depth_range"], N_samples, inv_uniform, det, jitter)
-    out, out_dy, out_st, aux = _render_pass(ray_batch, featmaps[0], featmaps[2], pts, z, s, t, fidx,
-                                            [int(o) for o in time_offset[0]], num_vv,
-                                            model.net_coarse_dy, model.net_coarse_st, model.motion_mlp,
-                                            basis, 6, 1, want_vanilla_st=True, want_aux=True)
-    ret = {"outputs_coarse": None, "outputs_fine": None, "outputs_coarse_ref": out,
-           "outputs_coarse_ref_dy": out_dy, "outputs_coarse_st": out_st}
-    if is_train:
-      ret.update(_cross_time(ray_batch, featmaps[1], pts, z, aux, fidx, int(frame_idx[1]),
-                             _scalar(time_embedding[1].float()), [int(o) for o in time_offset[1]],
-                             num_vv, model, basis, args.occ_weights_mode, out, out_dy))
+    with torch.no_grad():
+      return _render_mono(frame_idx, time_embedding, time_offset, ray_batch, model, featmaps, N_samples, args,
+                          inv_uniform, det, is_train, num_vv, jitter, False)
+
+
+def _render_mono(frame_idx, time_embedding, time_offset, ray_batch, model, featmaps, N_samples, args, inv_uniform,
+                 det, is_train, num_vv, jitter, train):
+  """render_rays_mono on one batch of rays.  `train`: the stages that gradients pass through are
+  `torch.autograd.Function`s over the forward/backward kernels (dynibar_b200/autograd.py), so gradients reach the
+  parameters of motion_mlp / net_coarse_dy / net_coarse_st and the feature maps.  Training precision (the
+  library-wide setting / `precision=`): "bf16" runs the products of the three networks, forward and backward, on
+  tcgen05 (bf16 operands, fp32 accumulation, fp32 master weights and gradients); "fp32" = SIMT products."""
+  t = _scalar(time_embedding[0].float())
+  ray_batch, hb = _with_host_copies(ray_batch, model, ("trajectory_basis",))
+  basis = hb["trajectory_basis"]
+  fidx = int(frame_idx[0])
+  pts, z, s = sample_along_camera_ray(ray_batch["ray_o"], ray_batch["ray_d"], ray_batch["depth_range"], N_samples,
+                                      inv_uniform, det, jitter)
+  out, out_dy, out_st, aux = _render_pass(ray_batch, featmaps[0], featmaps[2], pts, z, s, t, fidx,
+                                          [int(o) for o in time_offset[0]], num_vv, model.net_coarse_dy,
+                                          model.net_coarse_st, model.motion_mlp, basis, 6, 1, train=train,
+                                          want_vanilla_st=True)
+  ret = {"outputs_coarse": None, "outputs_fine": None, "outputs_coarse_ref": out,
+         "outputs_coarse_ref_dy": out_dy, "outputs_coarse_st": out_st}
+  if is_train:
+    ret.update(_cross_time(ray_batch, featmaps[1], pts, z, aux, fidx, int(frame_idx[1]),
+                           _scalar(time_embedding[1].float()), [int(o) for o in time_offset[1]], num_vv, model,
+                           basis, args.occ_weights_mode, out, out_dy, train))
   return ret
 
 
 def _cross_time(ray_batch, feat_anchor, pts, z, aux, ref_idx, anc_idx, t_anc, anchor_offsets, num_vv,
-                model, basis, occ_mode, out_ref, out_ref_dy):
+                model, basis, occ_mode, out_ref, out_ref_dy, train):
   """Cross-time rendering for temporal consistency (render_ray.py:1099-1270)."""
   coeff = aux["coeff"]
-  sf_seq = traj_deltas(coeff, basis, [ref_idx + o for o in (-2, -1, 0, 1, 2, 3)],
-                       [ref_idx + o - 1 for o in (-2, -1, 0, 1, 2, 3)])
-  pts_anchor = displaced_points(pts, coeff, basis, ref_idx, [anc_idx - ref_idx])[0]  # :1109-1112
-  coeff_a = motion_coefficients(model.motion_mlp, pts_anchor, t_anc)                 # :1126-1127
-  seq_a = displaced_points(pts_anchor, coeff_a, basis, anc_idx, anchor_offsets, num_vv)  # :1149-1176
-  keep = [(i, anc_idx + o - ref_idx) for i, o in enumerate(anchor_offsets)
+  sf_seq = _deltas(train, coeff, basis, [ref_idx + o for o in (-2, -1, 0, 1, 2, 3)],
+                   [ref_idx + o - 1 for o in (-2, -1, 0, 1, 2, 3)])
+  pts_anchor = _displace(train, pts, coeff, basis, ref_idx, [anc_idx - ref_idx])[0]  # :1109-1112
+  coeff_a = _coefficients(train, model.motion_mlp, pts_anchor, t_anc)                 # :1126-1127
+  seq_a = _displace(train, pts_anchor, coeff_a, basis, anc_idx, anchor_offsets, num_vv)  # :1149-1176
+  kept = [(i, anc_idx + o - ref_idx) for i, o in enumerate(anchor_offsets)
           if -3 <= anc_idx + o - ref_idx <= 3]
-  pts_traj_anchor = seq_a[[i for i, _ in keep]]
-  pts_traj_ref = displaced_points(pts, coeff, basis, ref_idx, [ro for _, ro in keep])
-  cam = ray_batch["camera"]
-  V_a = ray_batch["anchor_src_cameras"].shape[1]
-  if _prec() == _lib.PREC_BF16 and USE_FUSED and V_a <= 16:
-    raw_a, m_a = net_dynamic_fused(model.net_coarse_dy, pts_anchor, seq_a, aux["ray_dir"], cam,
-                                   ray_batch["anchor_src_rgbs"], ray_batch["anchor_src_cameras"],
-                                   featmaps_channels_last(feat_anchor), t_anc)
-  else:
-    f_a, _, m_a = project_gather(pts, seq_a, cam, ray_batch["anchor_src_rgbs"],
-                                 ray_batch["anchor_src_cameras"], feat_anchor)
-    raw_a = net_dynamic_forward(model.net_coarse_dy, pts_anchor, f_a, aux["ray_dir"], m_a, t_anc)
-  m_st = aux["m_st"]
+  pts_traj_anchor = seq_a[[i for i, _ in kept]]
+  pts_traj_ref = _displace(train, pts, coeff, basis, ref_idx, [ro for _, ro in kept])
+  cams_a = ray_batch["anchor_src_cameras"]
+  raw_a, m_a = _dynamic_branch(train, _fused(train, cams_a), model.net_coarse_dy, pts, pts_anchor, seq_a,
+                               aux["ray_dir"], ray_batch["camera"], ray_batch["anchor_src_rgbs"], cams_a,
+                               feat_anchor, t_anc)
   # anchor samples count when ANY view sees them (render_ray.py:1198-1200)
-  out_a = _composite(raw_a, aux["raw_st"], z, m_a, V_a, 0, m_st, m_st.shape[2], 1)
-  out_a_dy = _composite_vanilla(raw_a, z, m_a, V_a, 0)
+  out_a = ag.composite(raw_a, aux["raw_st"], z, m_a, aux["m_st"], 0, 1)
+  out_a_dy = ag.composite_vanilla(raw_a, z, m_a, 0)
   if occ_mode == 0:
     key = "weights_dy" if abs(ref_idx - anc_idx) > 1 else "weights"
   elif occ_mode == 1:
@@ -662,6 +679,7 @@ def _cross_time(ray_batch, feat_anchor, pts, z, aux, ref_idx, anc_idx, t_anc, an
     key = "weights"
   else:
     raise NotImplementedError
+  # detached in the reference (:1222, :1254)
   out_a["occ_weights"], out_a["occ_weight_map"] = occlusion_weights(out_ref[key], out_a[key])
   out_a["pts_traj_ref"] = pts_traj_ref
   out_a["pts_traj_anchor"] = pts_traj_anchor
@@ -671,9 +689,6 @@ def _cross_time(ray_batch, feat_anchor, pts, z, aux, ref_idx, anc_idx, t_anc, an
   return {"outputs_coarse_anchor": out_a, "outputs_coarse_anchor_dy": out_a_dy}
 
 
-# ---------------------------------------------------------------------------
-# f2: differentiable render_rays_mono (training step)
-# ---------------------------------------------------------------------------
 # (point, view) rows one training call of a network may hold (csrc/nets_f32.cu: net_rows_per_chunk; the training
 # forward keeps every activation of ONE internal chunk); larger ray batches are rendered in slices
 TRAIN_ROWS_LIMIT = 4194304
@@ -682,24 +697,24 @@ _RAY_AXIS1 = ("render_flows", "pts_traj_ref", "pts_traj_anchor", "sf_seq")  # [n
 
 def _render_mono_train_chunked(frame_idx, time_embedding, time_offset, ray_batch, model, featmaps, N_samples, args,
                                inv_uniform, det, is_train, num_vv, jitter):
-  """Slices the rays so that no network call exceeds TRAIN_ROWS_LIMIT rows and concatenates the per-slice output
-  dicts along their ray axis (autograd sees one graph; gradients accumulate over the slices)."""
+  """Slices the rays so that no network call exceeds TRAIN_ROWS_LIMIT rows, renders each slice with
+  `_render_mono(..., train=True)` and concatenates the per-slice output dicts along their ray axis (autograd sees
+  one graph; gradients accumulate over the slices)."""
   R = ray_batch["ray_o"].shape[0]
   vmax = max(ray_batch[k].shape[1] for k in ("src_cameras", "static_src_cameras", "anchor_src_cameras")
              if k in ray_batch and (is_train or k != "anchor_src_cameras"))
   per = max(1, TRAIN_ROWS_LIMIT // (N_samples * vmax))
   if R <= per:
-    return _render_mono_train(frame_idx, time_embedding, time_offset, ray_batch, model, featmaps, N_samples, args,
-                              inv_uniform, det, is_train, num_vv, jitter)
+    return _render_mono(frame_idx, time_embedding, time_offset, ray_batch, model, featmaps, N_samples, args,
+                        inv_uniform, det, is_train, num_vv, jitter, True)
   parts = []
   for lo in range(0, R, per):
     hi = min(R, lo + per)
     rb = dict(ray_batch)
     for k in ("ray_o", "ray_d", "uv_grid"):
       rb[k] = ray_batch[k][lo:hi]
-    parts.append(_render_mono_train(frame_idx, time_embedding, time_offset, rb, model, featmaps, N_samples, args,
-                                    inv_uniform, det, is_train, num_vv,
-                                    None if jitter is None else jitter[lo:hi]))
+    parts.append(_render_mono(frame_idx, time_embedding, time_offset, rb, model, featmaps, N_samples, args,
+                              inv_uniform, det, is_train, num_vv, None if jitter is None else jitter[lo:hi], True))
   ret = {}
   for name, first in parts[0].items():
     if first is None:
@@ -707,96 +722,4 @@ def _render_mono_train_chunked(frame_idx, time_embedding, time_offset, ray_batch
       continue
     ret[name] = OrderedDict((k, torch.cat([p[name][k] for p in parts], 1 if k in _RAY_AXIS1 else 0))
                             for k in first)
-  return ret
-
-
-def _render_mono_train(frame_idx, time_embedding, time_offset, ray_batch, model, featmaps, N_samples, args,
-                       inv_uniform, det, is_train, num_vv, jitter):
-  """render_rays_mono (render_ray.py:870-1277) with autograd: the same sequence as the reference, every stage a
-  `torch.autograd.Function` over the forward/backward kernels (dynibar_b200/autograd.py).  Gradients reach
-  the parameters of motion_mlp / net_coarse_dy / net_coarse_st and the feature maps.  torch itself only
-  concatenates the time column, zeroes the last samples' coefficients, slices and detaches.  Precision (the
-  library-wide setting / `precision=`): "bf16" runs the products of the three networks, forward and backward, on
-  tcgen05 (bf16 operands, fp32 accumulation, fp32 master weights and gradients); "fp32" = SIMT products."""
-  from dynibar_b200 import autograd as ag
-  t = _scalar(time_embedding[0].float())
-  rb, hb = _with_host_copies(ray_batch, model, ("trajectory_basis",))
-  basis = hb["trajectory_basis"]  # host [T, nb]; rows indexed like the reference (negative indices wrap)
-  fidx = int(frame_idx[0])
-  ref_offsets = [int(o) for o in time_offset[0]]
-  with torch.no_grad():
-    pts, z, s = sample_along_camera_ray(rb["ray_o"], rb["ray_d"], rb["depth_range"], N_samples, inv_uniform, det,
-                                        jitter)
-    ref_plucker = compute_ref_plucker_coordinate(rb["ray_o"], rb["ray_d"])
-    src_plucker = compute_src_plucker_coordinate(pts, rb["static_src_cameras"])
-  ray_dir = ref_plucker[:, :3]
-  dev = dev_of(pts)
-  R, S = pts.shape[:2]
-  n_last = int(round(S * 0.1))
-  keep = torch.ones(1, S, 1, device=dev)
-  if n_last > 0:
-    keep[:, S - n_last:] = 0.0
-  zero = torch.zeros_like(basis[0])
-
-  def rows(pairs):  # D[i] = basis[a_i] - basis[b_i] (b = None: zero row), on the device
-    return torch.stack([basis[a] - basis[b] if a is not None else zero for a, b in pairs]).to(dev)
-
-  def coeffs(p, tt):  # model.motion_mlp(cat[p, t]) with the last samples zeroed (:957-958, :1126-1127)
-    xyzt = torch.cat([p, torch.full((R, S, 1), tt, device=dev)], dim=-1)
-    return ag.motion_mlp(model.motion_mlp, xyzt) * keep
-
-  coeff = coeffs(pts, t)
-  seq = ag.traj_combine(coeff, rows([(fidx + o, fidx) for o in ref_offsets] + [(None, None)] * num_vv), pts)
-  cam = rb["camera"]
-  f_dy, _, m_dy = ag.project_gather(pts, seq, cam, rb["src_rgbs"], rb["src_cameras"], featmaps[0])
-  f_st, rd_st, m_st = ag.project_gather(pts, None, cam, rb["static_src_rgbs"], rb["static_src_cameras"],
-                                        featmaps[2])
-  raw_dy = ag.net_dynamic(model.net_coarse_dy, pts, f_dy, ray_dir, m_dy, t)
-  raw_st = ag.net_static(model.net_coarse_st, pts, ref_plucker, src_plucker, f_st, rd_st, m_st)
-  out = ag.composite(raw_dy, raw_st, z, m_dy, m_st, 1, 1)
-  out_st = ag.composite_vanilla(raw_st, z, m_st, 1)
-  out_dy = ag.composite_vanilla(raw_dy, z, m_dy, 1)
-  out["render_flows"] = ag.optical_flow(out["weights"], seq[:6], rb["src_cameras"][:, :6], rb["uv_grid"])
-  out["s_vals"] = s
-  with torch.no_grad():  # :1086-1096, detached in the reference
-    _, out["exp_sf"] = _flow_sceneflow(out["weights"], seq, rb["src_cameras"], rb["uv_grid"], coeff, basis, fidx,
-                                       1, 1)
-  ret = {"outputs_coarse": None, "outputs_fine": None, "outputs_coarse_ref": out,
-         "outputs_coarse_ref_dy": out_dy, "outputs_coarse_st": out_st}
-  if not is_train:
-    return ret
-  # ---- cross-time rendering for temporal consistency (:1099-1270)
-  anc = int(frame_idx[1])
-  t_anc = _scalar(time_embedding[1].float())
-  anchor_offsets = [int(o) for o in time_offset[1]]
-  sf_seq = ag.traj_combine(coeff, rows([(fidx + o, fidx + o - 1) for o in (-2, -1, 0, 1, 2, 3)]))
-  pts_anchor = ag.traj_combine(coeff, rows([(anc, fidx)]), pts)[0]
-  coeff_a = coeffs(pts_anchor, t_anc)
-  seq_a = ag.traj_combine(coeff_a, rows([(anc + o, anc) for o in anchor_offsets] + [(None, None)] * num_vv),
-                          pts_anchor)
-  kept = [(i, anc + o - fidx) for i, o in enumerate(anchor_offsets) if -3 <= anc + o - fidx <= 3]
-  pts_traj_anchor = seq_a[[i for i, _ in kept]]
-  pts_traj_ref = ag.traj_combine(coeff, rows([(fidx + ro, fidx) for _, ro in kept]), pts)
-  f_a, _, m_a = ag.project_gather(pts, seq_a, cam, rb["anchor_src_rgbs"], rb["anchor_src_cameras"], featmaps[1])
-  raw_a = ag.net_dynamic(model.net_coarse_dy, pts_anchor, f_a, ray_dir, m_a, t_anc)
-  # anchor samples count when ANY view sees them (render_ray.py:1198-1200)
-  out_a = ag.composite(raw_a, raw_st, z, m_a, m_st, 0, 1)
-  out_a_dy = ag.composite_vanilla(raw_a, z, m_a, 0)
-  occ_mode = args.occ_weights_mode
-  if occ_mode == 0:
-    key = "weights_dy" if abs(fidx - anc) > 1 else "weights"
-  elif occ_mode == 1:
-    key = "weights_dy"
-  elif occ_mode == 2:
-    key = "weights"
-  else:
-    raise NotImplementedError
-  with torch.no_grad():  # detached in the reference (:1222, :1254)
-    out_a["occ_weights"], out_a["occ_weight_map"] = occlusion_weights(out[key], out_a[key])
-    out_a_dy["occ_weights"], out_a_dy["occ_weight_map"] = occlusion_weights(out_dy["weights"], out_a_dy["weights"])
-  out_a["pts_traj_ref"] = pts_traj_ref
-  out_a["pts_traj_anchor"] = pts_traj_anchor
-  out_a["sf_seq"] = sf_seq
-  ret["outputs_coarse_anchor"] = out_a
-  ret["outputs_coarse_anchor_dy"] = out_a_dy
   return ret

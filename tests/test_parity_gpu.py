@@ -118,7 +118,8 @@ def test_motion_mlp_forward_module_call(rr):
 
 
 @pytest.mark.parametrize("S", [16, 64, 128, 100])
-def test_composite(rr, S):
+def test_composite_dicts(rr, S):
+  from dynibar_b200 import autograd as ag
   torch.manual_seed(S)
   R, Va, Vb = 53, 7, 5
   raw_a, raw_b = torch.randn(R, S, 4), torch.randn(R, S, 4)
@@ -131,12 +132,12 @@ def test_composite(rr, S):
   mb = (torch.rand(R, S, Vb) > 0.6).float()
   ma[7] = 0
   want = orc.composite(raw_a, raw_b, z, ma.sum(2) > 1, mb.sum(2) > 1)
-  got = rr._composite(_dev(raw_a), _dev(raw_b), _dev(z), _dev(ma), Va, 1, _dev(mb), Vb, 1)
+  got = ag.composite(_dev(raw_a), _dev(raw_b), _dev(z), _dev(ma), _dev(mb), 1, 1)
   assert list(got.keys()) == list(want.keys())
   for k in want:
     assert_close_frac(k, got[k], want[k], rtol=1e-5, atol=1e-6)
   want = orc.composite_vanilla(raw_a, z, ma.sum(2) > 0)
-  got = rr._composite_vanilla(_dev(raw_a), _dev(z), _dev(ma), Va, 0)
+  got = ag.composite_vanilla(_dev(raw_a), _dev(z), _dev(ma), 0)
   assert list(got.keys()) == list(want.keys())
   for k in want:
     assert_close_frac(k, got[k], want[k], rtol=1e-5, atol=1e-6)

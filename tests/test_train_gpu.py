@@ -203,14 +203,21 @@ _TRAIN_KEYS = {
 }
 
 
-@pytest.mark.parametrize("name,prec", [("mono_train", "fp32"), ("mono_train_near", "fp32"), ("mono_train", "bf16")])
-def test_render_rays_mono_training_step_matches_oracle_autograd(name, prec):
+# S4: with 4 samples per ray round(0.1 * 4) = 0, and the reference's x[:, -0:] zeroes the motion coefficients of every
+# sample.  Without anti-alias pooling: with it, torch's own fp32 autograd of this 4-sample rig is 0.7 % away from its
+# fp64 autograd for the static net's attention weights, above the bar below; without it, under 0.1 % for every tensor.
+@pytest.mark.parametrize("name,prec,over", [("mono_train", "fp32", {}), ("mono_train_near", "fp32", {}),
+                                            ("mono_train", "bf16", {}),
+                                            ("mono_train", "fp32", dict(N_samples=4, anti_alias_pooling=0))],
+                         ids=["mono_train-fp32", "mono_train_near-fp32", "mono_train-bf16", "mono_train-fp32-S4"])
+def test_render_rays_mono_training_step_matches_oracle_autograd(name, prec, over):
   """The whole differentiable path: loss = sum of randomly weighted differentiable outputs of
   render_rays_mono(is_train=True); d loss / d (every parameter of motion_mlp, net_coarse_dy, net_coarse_st and the
   three feature maps) against torch autograd through the oracle."""
   from dynibar_b200 import render_ray as rr
   from dynibar_b200.projection import Projector
-  cfg = dict(scenes.GOLDEN_CONFIGS[name])
+  cfg = dict(scenes.GOLDEN_CONFIGS[name], **over)
+  motion_off = int(round(0.1 * cfg["N_samples"])) == 0  # every sample's motion coefficients are zeroed
   if prec == "bf16":
     cfg["rays"] = 96  # >= 2048 (point, view) rows per product: the tensor-core kernels take over
   batch, feat_c, _, frame, t, offs, model, args = scenes.build(cfg)
@@ -253,6 +260,8 @@ def test_render_rays_mono_training_step_matches_oracle_autograd(name, prec):
                    ("motion_mlp", om.motion_mlp)):
     for k, p in getattr(m_dev, mname).named_parameters():
       assert p.grad is not None, (mname, k)
+      if mname == "motion_mlp" and motion_off:
+        assert not p.grad.any(), (mname, k)
       if mname == "net_coarse_st" and k == "s":
         # ill-conditioned in fp32 on this rig (far samples: cos ~ 1 for every view, so the pooling weights are
         # (e - min e) / (sum + 1e-8) with sum ~ 1e-6): torch's own fp32 autograd differs from its fp64 autograd by

@@ -10,8 +10,9 @@ from dynibar_b200 import render_ray as rr
 
 
 def _fake_train(frame_idx, time_embedding, time_offset, ray_batch, model, featmaps, N_samples, args, inv_uniform, det,
-                is_train, num_vv, jitter):
+                is_train, num_vv, jitter, train=True):
   """Stands in for the CUDA path: every output is a per-ray function of ray_o, in the reference's layouts."""
+  assert train
   o = ray_batch["ray_o"]
   R = o.shape[0]
   s = o.sum(-1)
@@ -26,8 +27,8 @@ def _fake_train(frame_idx, time_embedding, time_offset, ray_batch, model, featma
   return {"outputs_coarse": None, "outputs_fine": None, "outputs_coarse_ref": out, "outputs_coarse_anchor": anchor}
 
 
-def test_ray_slices_are_merged_along_the_ray_axis(monkeypatch):
-  monkeypatch.setattr(rr, "_render_mono_train", _fake_train)
+def test_training_slices_are_merged_along_the_ray_axis(monkeypatch):
+  monkeypatch.setattr(rr, "_render_mono", _fake_train)
   g = torch.Generator().manual_seed(0)
   R, S, V = 23, 4, 3
   batch = {"ray_o": torch.randn(R, 3, generator=g), "ray_d": torch.randn(R, 3, generator=g),
